@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W [--workload C2]   # this repo's CUDA path (default: C2, the headline)
     python bench.py --impl reference --gpus N --steps K ...          # the reference algorithm on the host cores
+    python bench.py ... --dump-outputs DIR                           # also write a sample of the last step's result
 
 Workloads (BASELINE.json `configs`, SURVEY.md section 8d):
   C1     PolyBenchmark forwardNtt, N=4096, one 55-bit modulus (Benchmarks/PolyBenchmark/PolyBenchmark.swift:148-158)
@@ -17,7 +18,9 @@ Workloads (BASELINE.json `configs`, SURVEY.md section 8d):
 A "step" = one pass of the hot path over one batch of synthetic input.  `value` is device-resident throughput (inputs in
 HBM before the clock starts, CUDA events on the launch stream, max over ranks); `e2e` is the same work through the
 host-pointer C-ABI call with pinned host buffers (H2D + D2H inside the clock).  C4/C5 are host-API workloads (the
-query arrives from the host every time): there `value` and `e2e` are the same measurement.
+query arrives from the host every time): there `value` and `e2e` are the same measurement, and a step is one query on
+each of the 8 concurrent host threads (C4) or one batch of 16 query vectors (C5).  Every timed loop runs --steps
+iterations: the headline, `e2e` and the relinearize extras; only the roofline's lone-kernel timing is a fixed 20 launches.
 """
 from __future__ import annotations
 
@@ -62,6 +65,7 @@ WORKLOADS = {
 BUTTERFLY_PIPE_PEAK = {"value": 3.3, "unit": "butterflies/clk/SM",
                        "source": "profiles/r02_microbench_pipes.txt (Cooley-Tukey / Gentleman-Sande Shoup butterfly alone: "
                                  "3.2-3.4 at 4-16 warps per scheduler, multiply pipe 97-98 % busy)"}
+DUMP_BYTES = 48 << 20  # size of the --dump-outputs sample (float32 limbs)
 
 
 def workload_params(name):
@@ -367,6 +371,21 @@ class Harness:
         torch.cuda.synchronize()
         return k0.elapsed_time(k1) / reps
 
+    def dump(self, name, result):
+        """--dump-outputs DIR: a fixed, seeded sample of the units (first axis) of `result` as DIR/<name>.npy, rank 0 only.
+        Residues reach 62 bits and float64 holds 53 exactly, so each residue is written as its four 16-bit limbs (least
+        significant first, a trailing axis of 4) in float32: exact, and a change in any bit of a residue shows as a
+        difference of at least 1."""
+        out_dir = self.args.dump_outputs
+        if not out_dir or self.rank != 0:
+            return
+        count = min(result.shape[0], max(1, DUMP_BYTES // (result[0].numel() * 4 * 4)))
+        idx = np.sort(np.random.default_rng(0).choice(result.shape[0], count, replace=False))
+        sample = result[self.torch.from_numpy(idx).to(result.device)].cpu().numpy().view(np.uint64)
+        limbs = (sample[..., None] >> np.arange(0, 64, 16, dtype=np.uint64)) & np.uint64(0xFFFF)
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, f"{name}.npy"), limbs.astype(np.float32))
+
     def finish(self):
         if self.world > 1:
             self.dist.destroy_process_group()
@@ -422,13 +441,14 @@ def run_ntt(h, name):
         h.check(h.lib.hecuda_ntt_forward_device(ctx._h, hecuda.BASE_Q, data.data_ptr(), 1, batch, h.stream.cuda_stream))
 
     ms, launches, clocks = h.timed(step, args.steps, args.warmup)
+    h.dump("ntt", data)
     value = h.world * batch * args.steps / (ms / 1e3)
     roofline = ntt_roofline(h, ctx, hecuda.BASE_Q, 1, batch, n, f"ntt_rows_kernel<{n.bit_length() - 1}, forward> (one NARROW modulus)")
     e2e = None
     if not args.no_e2e:
         hb = hecuda.PinnedBuffer((batch, 1, n))
         hb.array[...] = data.cpu().numpy().view(np.uint64)
-        steps = max(2, min(args.steps, 5))
+        steps = args.steps
         h.check(h.lib.hecuda_ntt_forward(ctx._h, hecuda.BASE_Q, hb.array.ctypes.data, 1, batch))
         h.barrier()
         t0 = time.perf_counter()
@@ -480,6 +500,7 @@ def run_mul(h, name):
                                                  h.stream.cuda_stream))
 
     ms, launches, clocks = h.timed(step, args.steps, args.warmup)
+    h.dump("product", out)
     value = h.world * batch * args.steps / (ms / 1e3)
     peak, _ = hbm_peak()
     R = 2 * L + 1
@@ -521,7 +542,7 @@ def run_mul(h, name):
             h.check(h.lib.hecuda_bfv_relinearize_device(ctx._h, evk._h, out.data_ptr(), L, relin_out.data_ptr(), batch,
                                                         h.stream.cuda_stream))
 
-        reps = max(3, min(args.steps, 10))
+        reps = args.steps
         for label, fn in (("relinearize_per_s", relin_step), ("multiply_relinearize_per_s", lambda: (step(), relin_step()))):
             tt, _, _ = h.timed(fn, reps, 2, sample_clocks=False)
             extra[label] = h.world * batch * reps / (tt / 1e3)
@@ -539,7 +560,7 @@ def run_mul(h, name):
         ho = hecuda.PinnedBuffer((batch, 3, L, n), dt_host)
         hl.array[...] = lhs.cpu().numpy().view(np.uint64)
         hr.array[...] = rhs.cpu().numpy().view(np.uint64)
-        steps = max(2, min(args.steps, 5))
+        steps = args.steps
 
         def host_mul():
             if word32:
@@ -611,6 +632,7 @@ def run_relin(h, name):
         h.check(h.lib.hecuda_bfv_mod_switch_down_device(ctx._h, relin.data_ptr(), 2, L, down.data_ptr(), mine, h.stream.cuda_stream))
 
     ms, launches, clocks = h.timed(step, args.steps, args.warmup)
+    h.dump("mod_switched", down)
     value = total * args.steps / (ms / 1e3)
     peak, _ = hbm_peak()
     roofline = ntt_roofline(h, ctx, hecuda.BASE_KEYSWITCH, K, min(mine, 256), n,
@@ -630,7 +652,7 @@ def run_relin(h, name):
         hin, hmid = hecuda.PinnedBuffer((eb, 3, L, n)), hecuda.PinnedBuffer((eb, 2, L, n))
         hout = hecuda.PinnedBuffer((eb, 2, L - 1, n))
         hin.array[...] = ct3[:eb].cpu().numpy().view(np.uint64)
-        steps = max(2, min(args.steps, 3))
+        steps = args.steps
 
         def host_step():
             hecuda.Bfv.relinearize(ctx, hin.array, evk, out=hmid.array)
@@ -690,12 +712,11 @@ def run_app(args, name):
     if kind == "pir":
         import bench_pir
 
-        threads = 8
-        per_thread = max(10, 6 * args.steps)
-        r = bench_pir.run(1 << 20, 64, threads, per_thread, cpu=not args.no_cpu_baseline)
+        threads = 8  # one step = one query on each of the `threads` concurrent host threads
+        r = bench_pir.run(1 << 20, 64, threads, args.steps, cpu=not args.no_cpu_baseline)
         if r is None:
             return
-        value, steps = r["value"], threads * per_thread
+        value, steps = r["value"], args.steps
         ms = r["concurrent_s"] * 1e3
         scan = r["db_scan_gbs_at_value"] / world
         roofline = {"bound": "hbm", "kernel": "inner_product_plain_kernel (first-dimension scan of the resident database)",
@@ -707,7 +728,7 @@ def run_app(args, name):
     else:
         import bench_pnns
 
-        reps = max(3, min(args.steps, 10))
+        reps = args.steps  # one step = one batch of 16 query vectors
         r = bench_pnns.run(100000, 512, 16, reps, cpu=not args.no_cpu_baseline)
         if r is None:
             return
@@ -738,12 +759,18 @@ def main():
     ap.add_argument("--batch", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a seeded sample of the last step's result to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
+    kind = WORKLOADS[args.workload][0]
+    if args.dump_outputs and (args.impl == "reference" or kind in ("pir", "pnns")):
+        ap.error("--dump-outputs covers the GPU arm of the device-resident workloads (all but C4 and C5)")
 
     if args.impl == "reference":
         return run_reference(args)
-    kind = WORKLOADS[args.workload][0]
     if kind in ("pir", "pnns"):
         return run_app(args, args.workload)
 
