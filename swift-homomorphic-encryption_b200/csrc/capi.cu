@@ -15,6 +15,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
 #include <map>
 #include <memory>
 #include <mutex>
@@ -198,22 +199,30 @@ size_t inner_product_scratch_words(const Context &c, int64_t pairs) {
 
 namespace {
 
-// The u32 entry points (Bfv<UInt32> contexts) run the same bodies: the calling thread marks its host buffers as uint32
-// for the duration of the call and the pipeline widens after the H2D copy / narrows before the D2H copy.
-thread_local bool tl_io32 = false;
-struct Io32Scope {
-    Io32Scope() { tl_io32 = true; }
-    ~Io32Scope() { tl_io32 = false; }
+// Where the buffers of a batched call live and how wide their words are.  Host64 / Host32 run the double-buffered host
+// pipeline; Host32 buffers hold uint32 words (Bfv<UInt32>), widened after each H2D copy and narrowed before each D2H
+// copy.  Device buffers are uint64 on the device, enqueued on the caller's stream.
+enum class Io { Host64, Host32, Device };
+
+// A caller buffer of `words_per_item` words per batch item.
+struct Operand {
+    const u64 *src;
+    size_t words_per_item;
+};
+
+// One chunk of a batched call: items [first, first + items) of the batch, on device buffers.
+struct Chunk {
+    u64 *scratch;  // the op's scratch words per item x items
+    const u64 *in[2];
+    u64 *out;
+    int64_t first, items;
+    cudaStream_t stream;
 };
 
 // Generic double-buffered host pipeline: for each chunk, copy inputs in, run `body`, copy outputs out.
-struct HostIo {
-    const u64 *src;  // host
-    size_t words_per_item;
-};
 template <class Body>
-int32_t host_pipeline(const hecuda_context *h, int64_t batch, int64_t chunk_hint, size_t scratch_words_per_item,
-                      const std::vector<HostIo> &inputs, u64 *host_out, size_t out_words_per_item, Body body) {
+int32_t host_pipeline(const hecuda_context *h, bool io32, int64_t batch, int64_t chunk_hint, size_t scratch_words_per_item,
+                      std::initializer_list<Operand> inputs, u64 *host_out, size_t out_words_per_item, Body body) {
     if (batch == 0) return HECUDA_OK;
     // `depth` stages in flight, each on its own stream: H2D of stage k+1.., kernels of stage k, D2H of stage k-1
     static const int depth = [] {
@@ -250,8 +259,7 @@ int32_t host_pipeline(const hecuda_context *h, int64_t batch, int64_t chunk_hint
         // Work on one workspace is ordered by its stream; buffers only ever grow (first `depth` iterations).
         // slot 0 = kernel scratch, slot 4 = staged inputs (back to back), slot 5 = staged output
         size_t in_words = 0;
-        for (const HostIo &io : inputs) in_words += io.words_per_item * (size_t)items;
-        const bool io32 = tl_io32;
+        for (const Operand &io : inputs) in_words += io.words_per_item * (size_t)items;
         const size_t out_words = out_words_per_item * (size_t)items;
         CK(w.reserve(0, scratch_words_per_item * (size_t)items));
         CK(w.reserve(4, in_words));
@@ -260,9 +268,10 @@ int32_t host_pipeline(const hecuda_context *h, int64_t batch, int64_t chunk_hint
             CK(w.reserve(6, in_words / 2 + inputs.size() * 2 + 2));
             CK(w.reserve(7, out_words / 2 + 2));
         }
-        std::vector<const u64 *> d_in;
+        Chunk c{w.buf[0], {nullptr, nullptr}, w.buf[5], done, items, w.stream};
         size_t off = 0, off32 = 0;
-        for (const HostIo &io : inputs) {
+        int i = 0;
+        for (const Operand &io : inputs) {
             const size_t words = io.words_per_item * (size_t)items;
             if (io32) {
                 u32 *raw = reinterpret_cast<u32 *>(w.buf[6]) + off32;
@@ -274,10 +283,10 @@ int32_t host_pipeline(const hecuda_context *h, int64_t batch, int64_t chunk_hint
                 CK(cudaMemcpyAsync(w.buf[4] + off, io.src + io.words_per_item * (size_t)done, words * sizeof(u64),
                                    cudaMemcpyHostToDevice, w.stream));
             }
-            d_in.push_back(w.buf[4] + off);
+            c.in[i++] = w.buf[4] + off;
             off += words;
         }
-        cudaError_t e = body(w, d_in, w.buf[5], items);
+        cudaError_t e = body(c);
         if (e != cudaSuccess) return cuda_fail(e, "kernel launch");
         if (io32) {
             CK(launch_narrow(w.buf[5], reinterpret_cast<u32 *>(w.buf[7]), (int64_t)out_words, w.stream));
@@ -290,6 +299,79 @@ int32_t host_pipeline(const hecuda_context *h, int64_t batch, int64_t chunk_hint
     }
     for (Workspace *w : ws) CK(wait_stream(w->stream));
     return HECUDA_OK;
+}
+
+// Runs `body` over a batch of `batch` items held in `io`'s buffers.  Host calls go through the host pipeline, which
+// stages at most `chunk_hint` items at a time.  Device calls enqueue on `stream` and do not synchronise (so they can
+// be captured in a graph): ops with scratch run in chunks of min(chunk_hint, batch) items over one stream-ordered
+// allocation, scratch-free ops run the whole batch in one pass.  `what` names a failed device launch.
+template <class Body>
+int32_t dispatch(const hecuda_context *h, Io io, void *stream, const char *what, int64_t batch, int64_t chunk_hint,
+                 size_t scratch_words_per_item, std::initializer_list<Operand> inputs, void *out, size_t out_words_per_item,
+                 Body body) {
+    if (io != Io::Device)
+        return host_pipeline(h, io == Io::Host32, batch, chunk_hint, scratch_words_per_item, inputs, (u64 *)out,
+                             out_words_per_item, body);
+    if (batch == 0) return HECUDA_OK;
+    cudaStream_t s = (cudaStream_t)stream;
+    const int64_t chunk = scratch_words_per_item ? std::max<int64_t>(1, std::min<int64_t>(chunk_hint, batch)) : batch;
+    u64 *scratch = nullptr;
+    if (scratch_words_per_item) CK(cudaMallocAsync(&scratch, scratch_words_per_item * (size_t)chunk * sizeof(u64), s));
+    cudaError_t e = cudaSuccess;
+    for (int64_t first = 0; first < batch && e == cudaSuccess; first += chunk) {
+        Chunk c{scratch, {nullptr, nullptr}, (u64 *)out + out_words_per_item * first, first,
+                std::min<int64_t>(chunk, batch - first), s};
+        int i = 0;
+        for (const Operand &io : inputs) c.in[i++] = io.src + io.words_per_item * first;
+        e = body(c);
+    }
+    if (scratch) {
+        const cudaError_t f = cudaFreeAsync(scratch, s);
+        if (e == cudaSuccess && f != cudaSuccess) return cuda_fail(f, "cudaFreeAsync(scratch, s)");
+    }
+    return e == cudaSuccess ? HECUDA_OK : cuda_fail(e, what);
+}
+
+// uint32 buffers need a context made by hecuda_context_create_u32 (its m~, gamma and Bsk).
+int32_t need_word32(const hecuda_context *h) {
+    if (!h || !h->ctx) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidContext: null context");
+    if (h->ctx->word_bits != 32) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidContext: not a Bfv<UInt32> context (hecuda_context_create_u32)");
+    return HECUDA_OK;
+}
+
+// The first check of every batched call: the Host32 precondition, then the context.
+int32_t check_io(const hecuda_context *h, Io io) {
+    if (io == Io::Host32) {
+        int32_t rc = need_word32(h);
+        if (rc) return rc;
+    }
+    return check_ctx(h);
+}
+
+// The evaluation key of a call is present (for relinearization: filled in) and belongs to the call's context.
+int32_t check_key(const hecuda_context *h, const hecuda_evk *k, bool relin) {
+    if (!k || (relin && !k->loaded)) return fail(HECUDA_ERR_MISSING_KEY, relin ? "missingRelinearizationKey" : "missingGaloisKey");
+    if (k->owner != h) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidContext: evaluation key belongs to another context");
+    return HECUDA_OK;
+}
+
+// 1 <= l <= L; `kind` is the error's prefix (invalidCiphertext / invalidPolyContext).
+int32_t check_level(const hecuda_context *h, int32_t l, const char *kind) {
+    if (l < 1 || l > h->ctx->L) return fail(HECUDA_ERR_INVALID_ARGUMENT, std::string(kind) + ": moduli_count out of range");
+    return HECUDA_OK;
+}
+
+// A batch size is not negative, and a non-empty batch has every buffer.
+int32_t check_batch(int64_t batch, std::initializer_list<const void *> buffers, const char *msg) {
+    bool missing = false;
+    for (const void *p : buffers) missing |= !p;
+    if (batch < 0 || (batch && missing)) return fail(HECUDA_ERR_INVALID_ARGUMENT, msg);
+    return HECUDA_OK;
+}
+
+// Items per host-pipeline stage for a scratch-free op: ~4 M words (32 MB) of `words_per_item`-word items per stage.
+int64_t stage_items(size_t words_per_item, size_t stage_words = (size_t)4 * 1024 * 1024) {
+    return std::max<int64_t>(1, (int64_t)(stage_words / std::max<size_t>(1, words_per_item)));
 }
 
 }  // namespace
@@ -485,142 +567,102 @@ int32_t hecuda_context_root_tables(const hecuda_context *h, uint64_t modulus, ui
 
 // ---------------------------------------------------------------- NTT
 
-static int32_t ntt_device(const hecuda_context *h, int32_t base, uint64_t *data, int32_t rows, int64_t polys,
-                          void *stream, bool inverse) {
-    int32_t rc = check_ctx(h);
-    if (rc) return rc;
-    if (polys < 0 || (!data && polys)) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalid data / poly_count");
+// In place: `items` items of `rows_per_item` rows (`words_per_item` words) each.
+static int32_t ntt_run(const hecuda_context *h, Io io, void *stream, const NttRowMap &map, void *data, size_t words_per_item,
+                       int64_t items, int64_t rows_per_item, bool inverse) {
+    const Context &c = *h->ctx;
+    return dispatch(h, io, stream, "ntt launch", items, stage_items(words_per_item), 0, {{(const u64 *)data, words_per_item}},
+                    data, words_per_item, [&](const Chunk &k) {
+                        return inverse ? launch_ntt_inverse(c, map, k.in[0], k.out, k.items * rows_per_item, kScalePlain, k.stream)
+                                       : launch_ntt_forward(c, map, k.in[0], k.out, k.items * rows_per_item, k.stream);
+                    });
+}
+static int32_t ntt(const hecuda_context *h, int32_t base, void *data, int32_t rows, int64_t polys, bool inverse, Io io,
+                   void *stream = nullptr) {
+    int32_t rc = check_io(h, io);
+    if (rc || (rc = check_batch(polys, {data}, "invalid data / poly_count"))) return rc;
     NttRowMap map;
     std::string err;
     if (!make_map(*h->ctx, base, rows, map, err)) return fail(HECUDA_ERR_INVALID_ARGUMENT, err);
-    cudaError_t e = inverse ? launch_ntt_inverse(*h->ctx, map, (u64 *)data, (u64 *)data, polys * rows, kScalePlain,
-                                                 (cudaStream_t)stream)
-                            : launch_ntt_forward(*h->ctx, map, (u64 *)data, (u64 *)data, polys * rows,
-                                                 (cudaStream_t)stream);
-    if (e != cudaSuccess) return cuda_fail(e, "ntt launch");
-    return HECUDA_OK;
+    return ntt_run(h, io, stream, map, data, (size_t)rows * h->ctx->n, polys, rows, inverse);
 }
 int32_t hecuda_ntt_forward_device(const hecuda_context *h, int32_t base, uint64_t *data, int32_t rows, int64_t polys,
                                   void *stream) {
-    return ntt_device(h, base, data, rows, polys, stream, false);
+    return ntt(h, base, data, rows, polys, false, Io::Device, stream);
 }
 int32_t hecuda_ntt_inverse_device(const hecuda_context *h, int32_t base, uint64_t *data, int32_t rows, int64_t polys,
                                   void *stream) {
-    return ntt_device(h, base, data, rows, polys, stream, true);
-}
-
-static int32_t ntt_host(const hecuda_context *h, const NttRowMap &map, uint64_t *data, size_t words_per_item,
-                        int64_t items, int64_t rows_per_item, bool inverse) {
-    const Context &c = *h->ctx;
-    std::vector<HostIo> in = {{(const u64 *)data, words_per_item}};
-    // NTT items are single polynomials: stage ~32 MB per pipeline step
-    const int64_t chunk = std::max<int64_t>(1, (int64_t)((size_t)4 * 1024 * 1024 / std::max<size_t>(1, words_per_item)));
-    return host_pipeline(h, items, chunk, 0, in, (u64 *)data, words_per_item,
-                         [&](Workspace &w, const std::vector<const u64 *> &d_in, u64 *d_out, int64_t n_items) {
-                             return inverse ? launch_ntt_inverse(c, map, d_in[0], d_out, n_items * rows_per_item, kScalePlain,
-                                                                 w.stream)
-                                            : launch_ntt_forward(c, map, d_in[0], d_out, n_items * rows_per_item,
-                                                                 w.stream);
-                         });
+    return ntt(h, base, data, rows, polys, true, Io::Device, stream);
 }
 int32_t hecuda_ntt_forward(const hecuda_context *h, int32_t base, uint64_t *data, int32_t rows, int64_t polys) {
-    int32_t rc = check_ctx(h);
-    if (rc) return rc;
-    if (polys < 0 || (!data && polys)) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalid data / poly_count");
-    NttRowMap map;
-    std::string err;
-    if (!make_map(*h->ctx, base, rows, map, err)) return fail(HECUDA_ERR_INVALID_ARGUMENT, err);
-    return ntt_host(h, map, data, (size_t)rows * h->ctx->n, polys, rows, false);
+    return ntt(h, base, data, rows, polys, false, Io::Host64);
 }
 int32_t hecuda_ntt_inverse(const hecuda_context *h, int32_t base, uint64_t *data, int32_t rows, int64_t polys) {
-    int32_t rc = check_ctx(h);
-    if (rc) return rc;
-    if (polys < 0 || (!data && polys)) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalid data / poly_count");
-    NttRowMap map;
-    std::string err;
-    if (!make_map(*h->ctx, base, rows, map, err)) return fail(HECUDA_ERR_INVALID_ARGUMENT, err);
-    return ntt_host(h, map, data, (size_t)rows * h->ctx->n, polys, rows, true);
-}
-// Stage-level BEHZ entry points over the reference's [Q, Bsk] (RnsTool.swift:324-331, 453-456), Coeff format.
-int32_t hecuda_rnstool_lift_q_to_qbsk(const hecuda_context *h, const uint64_t *polys, uint64_t *out, int64_t count) {
-    int32_t rc = check_ctx(h);
-    if (rc) return rc;
-    if (count < 0 || ((!polys || !out) && count)) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalid buffers / poly_count");
-    const Context &c = *h->ctx;
-    const size_t in_words = (size_t)c.L * c.n, out_words = (size_t)(2 * c.L + 1) * c.n;
-    std::vector<HostIo> in = {{(const u64 *)polys, in_words}};
-    return host_pipeline(h, count, std::max<int64_t>(1, (int64_t)((size_t)4 * 1024 * 1024 / out_words)), 0, in, (u64 *)out, out_words,
-                         [&](Workspace &w, const std::vector<const u64 *> &d_in, u64 *d_out, int64_t n_items) {
-                             return launch_lift(c, d_in[0], 1, d_out, 1, 0, n_items, w.stream, /*reference_base=*/true);
-                         });
-}
-int32_t hecuda_rnstool_floor_qbsk_to_q(const hecuda_context *h, const uint64_t *polys, uint64_t *out, int64_t count) {
-    int32_t rc = check_ctx(h);
-    if (rc) return rc;
-    if (count < 0 || ((!polys || !out) && count)) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalid buffers / poly_count");
-    const Context &c = *h->ctx;
-    const size_t in_words = (size_t)(2 * c.L + 1) * c.n, out_words = (size_t)c.L * c.n;
-    std::vector<HostIo> in = {{(const u64 *)polys, in_words}};
-    return host_pipeline(h, count, std::max<int64_t>(1, (int64_t)((size_t)4 * 1024 * 1024 / in_words)), 0, in, (u64 *)out, out_words,
-                         [&](Workspace &w, const std::vector<const u64 *> &d_in, u64 *d_out, int64_t n_items) {
-                             return launch_floor(c, d_in[0], d_out, n_items, w.stream, /*reference_base=*/true);
-                         });
+    return ntt(h, base, data, rows, polys, true, Io::Host64);
 }
 
-static int32_t ntt_rows_host(const hecuda_context *h, uint64_t modulus, uint64_t *data, int64_t rows, bool inverse) {
+// Stage-level BEHZ entry points over the reference's [Q, Bsk] (RnsTool.swift:324-331, 453-456), Coeff format.
+static int32_t lift_q_to_qbsk(const hecuda_context *h, const void *polys, void *out, int64_t count, Io io) {
+    int32_t rc = check_io(h, io);
+    if (rc || (rc = check_batch(count, {polys, out}, "invalid buffers / poly_count"))) return rc;
+    const Context &c = *h->ctx;
+    const size_t in_words = (size_t)c.L * c.n, out_words = (size_t)(2 * c.L + 1) * c.n;
+    return dispatch(h, io, nullptr, "liftQToQBsk", count, stage_items(out_words), 0, {{(const u64 *)polys, in_words}}, out,
+                    out_words, [&](const Chunk &k) {
+                        return launch_lift(c, k.in[0], 1, k.out, 1, 0, k.items, k.stream, /*reference_base=*/true);
+                    });
+}
+static int32_t floor_qbsk_to_q(const hecuda_context *h, const void *polys, void *out, int64_t count, Io io) {
+    int32_t rc = check_io(h, io);
+    if (rc || (rc = check_batch(count, {polys, out}, "invalid buffers / poly_count"))) return rc;
+    const Context &c = *h->ctx;
+    const size_t in_words = (size_t)(2 * c.L + 1) * c.n, out_words = (size_t)c.L * c.n;
+    return dispatch(h, io, nullptr, "floorQBskToQ", count, stage_items(in_words), 0, {{(const u64 *)polys, in_words}}, out,
+                    out_words, [&](const Chunk &k) {
+                        return launch_floor(c, k.in[0], k.out, k.items, k.stream, /*reference_base=*/true);
+                    });
+}
+int32_t hecuda_rnstool_lift_q_to_qbsk(const hecuda_context *h, const uint64_t *polys, uint64_t *out, int64_t count) {
+    return lift_q_to_qbsk(h, polys, out, count, Io::Host64);
+}
+int32_t hecuda_rnstool_floor_qbsk_to_q(const hecuda_context *h, const uint64_t *polys, uint64_t *out, int64_t count) {
+    return floor_qbsk_to_q(h, polys, out, count, Io::Host64);
+}
+
+static int32_t ntt_rows(const hecuda_context *h, uint64_t modulus, uint64_t *data, int64_t rows, bool inverse) {
     int32_t rc = check_ctx(h);
-    if (rc) return rc;
-    if (rows < 0 || (!data && rows)) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalid data / row_count");
+    if (rc || (rc = check_batch(rows, {data}, "invalid data / row_count"))) return rc;
     const int s = h->ctx->find_slot(modulus);
     if (s < 0) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidPolyContext: modulus is not part of this context");
-    return ntt_host(h, h->ctx->map_single(s), data, (size_t)h->ctx->n, rows, 1, inverse);
+    return ntt_run(h, Io::Host64, nullptr, h->ctx->map_single(s), data, (size_t)h->ctx->n, rows, 1, inverse);
 }
 int32_t hecuda_ntt_forward_rows(const hecuda_context *h, uint64_t modulus, uint64_t *data, int64_t rows) {
-    return ntt_rows_host(h, modulus, data, rows, false);
+    return ntt_rows(h, modulus, data, rows, false);
 }
 int32_t hecuda_ntt_inverse_rows(const hecuda_context *h, uint64_t modulus, uint64_t *data, int64_t rows) {
-    return ntt_rows_host(h, modulus, data, rows, true);
+    return ntt_rows(h, modulus, data, rows, true);
 }
 
 // ---------------------------------------------------------------- multiply
 
+static int32_t multiply(const hecuda_context *h, const void *lhs, const void *rhs, void *out, int64_t batch, Io io,
+                        void *stream = nullptr) {
+    int32_t rc = check_io(h, io);
+    if (rc || (rc = check_batch(batch, {lhs, rhs, out}, "invalidCiphertext: null buffer"))) return rc;
+    const Context &c = *h->ctx;
+    const size_t in_words = (size_t)2 * c.L * c.n, out_words = (size_t)3 * c.L * c.n;
+    return dispatch(h, io, stream, "multiply", batch, h->chunk, multiply_scratch_words(c),
+                    {{(const u64 *)lhs, in_words}, {(const u64 *)rhs, in_words}}, out, out_words, [&](const Chunk &k) {
+                        return multiply_chunk(c, k.scratch, k.in[0], k.in[1], k.out, k.items, k.stream);
+                    });
+}
 int32_t hecuda_bfv_multiply_device(const hecuda_context *h, const uint64_t *lhs, const uint64_t *rhs, uint64_t *out,
                                    int64_t batch, void *stream) {
-    int32_t rc = check_ctx(h);
-    if (rc) return rc;
-    if (batch < 0 || (batch && (!lhs || !rhs || !out))) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidCiphertext: null buffer");
-    if (batch == 0) return HECUDA_OK;
-    const Context &c = *h->ctx;
-    const size_t in_words = (size_t)2 * c.L * c.n, out_words = (size_t)3 * c.L * c.n;
-    const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(h->chunk, batch));
-    cudaStream_t s = (cudaStream_t)stream;
-    u64 *scratch = nullptr;  // stream-ordered scratch: no host synchronization, graph-capturable
-    CK(cudaMallocAsync(&scratch, multiply_scratch_words(c) * (size_t)chunk * sizeof(u64), s));
-    for (int64_t done = 0; done < batch; done += chunk) {
-        const int64_t items = std::min<int64_t>(chunk, batch - done);
-        cudaError_t e = multiply_chunk(c, scratch, (const u64 *)lhs + in_words * done, (const u64 *)rhs + in_words * done,
-                                       (u64 *)out + out_words * done, items, s);
-        if (e != cudaSuccess) {
-            cudaFreeAsync(scratch, s);
-            return cuda_fail(e, "multiply");
-        }
-    }
-    CK(cudaFreeAsync(scratch, s));
-    return HECUDA_OK;
+    return multiply(h, lhs, rhs, out, batch, Io::Device, stream);
 }
-
 int32_t hecuda_bfv_multiply(const hecuda_context *h, const uint64_t *lhs, const uint64_t *rhs, uint64_t *out,
                             int64_t batch) {
-    int32_t rc = check_ctx(h);
-    if (rc) return rc;
-    if (batch < 0 || (batch && (!lhs || !rhs || !out))) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidCiphertext: null buffer");
-    const Context &c = *h->ctx;
-    const size_t in_words = (size_t)2 * c.L * c.n, out_words = (size_t)3 * c.L * c.n;
-    std::vector<HostIo> in = {{(const u64 *)lhs, in_words}, {(const u64 *)rhs, in_words}};
-    return host_pipeline(h, batch, h->chunk, multiply_scratch_words(c), in, (u64 *)out, out_words,
-                         [&](Workspace &w, const std::vector<const u64 *> &d_in, u64 *d_out, int64_t items) {
-                             return multiply_chunk(c, w.buf[0], d_in[0], d_in[1], d_out, items, w.stream);
-                         });
+    return multiply(h, lhs, rhs, out, batch, Io::Host64);
 }
 
 // ---------------------------------------------------------------- evaluation key
@@ -677,105 +719,75 @@ int32_t hecuda_evk_device_buffer(hecuda_evk *k, void **device_ptr, uint64_t *byt
 
 // ---------------------------------------------------------------- relinearize / mod switch
 
-static int32_t check_relin(const hecuda_context *h, const hecuda_evk *k, const uint64_t *ct3, int32_t l, uint64_t *out,
-                           int64_t batch) {
-    int32_t rc = check_ctx(h);
-    if (rc) return rc;
-    if (!k || !k->loaded) return fail(HECUDA_ERR_MISSING_KEY, "missingRelinearizationKey");
-    if (k->owner != h) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidContext: evaluation key belongs to another context");
-    if (l < 1 || l > h->ctx->L) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidCiphertext: moduli_count out of range");
-    if (batch < 0 || (batch && (!ct3 || !out))) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidCiphertext: null buffer");
-    return HECUDA_OK;
+static int32_t relinearize(const hecuda_context *h, const hecuda_evk *k, const void *ct3, int32_t l, void *out,
+                           int64_t batch, Io io, void *stream = nullptr) {
+    int32_t rc = check_io(h, io);
+    if (rc || (rc = check_key(h, k, true)) || (rc = check_level(h, l, "invalidCiphertext")) ||
+        (rc = check_batch(batch, {ct3, out}, "invalidCiphertext: null buffer")))
+        return rc;
+    const Context &c = *h->ctx;
+    return dispatch(h, io, stream, "relinearize", batch, h->chunk, relinearize_scratch_words(c, l),
+                    {{(const u64 *)ct3, (size_t)3 * l * c.n}}, out, (size_t)2 * l * c.n, [&](const Chunk &ch) {
+                        return relinearize_chunk(c, ch.scratch, k->d_relin, ch.in[0], l, ch.out, ch.items, ch.stream);
+                    });
 }
-
 int32_t hecuda_bfv_relinearize_device(const hecuda_context *h, const hecuda_evk *k, const uint64_t *ct3, int32_t l,
                                       uint64_t *out, int64_t batch, void *stream) {
-    int32_t rc = check_relin(h, k, ct3, l, out, batch);
-    if (rc) return rc;
-    if (batch == 0) return HECUDA_OK;
-    const Context &c = *h->ctx;
-    const size_t in_words = (size_t)3 * l * c.n, out_words = (size_t)2 * l * c.n;
-    const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(h->chunk, batch));
-    cudaStream_t s = (cudaStream_t)stream;
-    u64 *scratch = nullptr;
-    CK(cudaMallocAsync(&scratch, relinearize_scratch_words(c, l) * (size_t)chunk * sizeof(u64), s));
-    for (int64_t done = 0; done < batch; done += chunk) {
-        const int64_t items = std::min<int64_t>(chunk, batch - done);
-        cudaError_t e = relinearize_chunk(c, scratch, k->d_relin, (const u64 *)ct3 + in_words * done, l,
-                                          (u64 *)out + out_words * done, items, s);
-        if (e != cudaSuccess) {
-            cudaFreeAsync(scratch, s);
-            return cuda_fail(e, "relinearize");
-        }
-    }
-    CK(cudaFreeAsync(scratch, s));
-    return HECUDA_OK;
+    return relinearize(h, k, ct3, l, out, batch, Io::Device, stream);
 }
-
 int32_t hecuda_bfv_relinearize(const hecuda_context *h, const hecuda_evk *k, const uint64_t *ct3, int32_t l,
                                uint64_t *out, int64_t batch) {
-    int32_t rc = check_relin(h, k, ct3, l, out, batch);
-    if (rc) return rc;
-    const Context &c = *h->ctx;
-    std::vector<HostIo> in = {{(const u64 *)ct3, (size_t)3 * l * c.n}};
-    return host_pipeline(h, batch, h->chunk, relinearize_scratch_words(c, l), in, (u64 *)out, (size_t)2 * l * c.n,
-                         [&](Workspace &w, const std::vector<const u64 *> &d_in, u64 *d_out, int64_t items) {
-                             return relinearize_chunk(c, w.buf[0], k->d_relin, d_in[0], l, d_out, items, w.stream);
-                         });
+    return relinearize(h, k, ct3, l, out, batch, Io::Host64);
 }
 
-static int32_t check_ms(const hecuda_context *h, const uint64_t *ct, int32_t polys, int32_t l, uint64_t *out,
-                        int64_t batch) {
-    int32_t rc = check_ctx(h);
+static int32_t mod_switch_down(const hecuda_context *h, const void *ct, int32_t polys, int32_t l, void *out, int64_t batch,
+                               Io io, void *stream = nullptr) {
+    int32_t rc = check_io(h, io);
     if (rc) return rc;
     if (polys < 1) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidCiphertext: poly_count");
     if (l < 2 || l > h->ctx->L)
         return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidPolyContext: modSwitchDown needs a next context (2 <= moduli_count <= L)");
-    if (batch < 0 || (batch && (!ct || !out))) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidCiphertext: null buffer");
-    return HECUDA_OK;
+    if ((rc = check_batch(batch, {ct, out}, "invalidCiphertext: null buffer"))) return rc;
+    const Context &c = *h->ctx;
+    const size_t in_words = (size_t)polys * l * c.n;
+    return dispatch(h, io, stream, "mod_switch", batch, stage_items(in_words), 0, {{(const u64 *)ct, in_words}}, out,
+                    (size_t)polys * (l - 1) * c.n, [&](const Chunk &k) {
+                        return launch_mod_switch(c, k.in[0], l, k.out, k.items * polys, k.stream);
+                    });
 }
-
 int32_t hecuda_bfv_mod_switch_down_device(const hecuda_context *h, const uint64_t *ct, int32_t polys, int32_t l,
                                           uint64_t *out, int64_t batch, void *stream) {
-    int32_t rc = check_ms(h, ct, polys, l, out, batch);
-    if (rc) return rc;
-    cudaError_t e = launch_mod_switch(*h->ctx, (const u64 *)ct, l, (u64 *)out, batch * polys, (cudaStream_t)stream);
-    if (e != cudaSuccess) return cuda_fail(e, "mod_switch");
-    return HECUDA_OK;
+    return mod_switch_down(h, ct, polys, l, out, batch, Io::Device, stream);
 }
-
 int32_t hecuda_bfv_mod_switch_down(const hecuda_context *h, const uint64_t *ct, int32_t polys, int32_t l, uint64_t *out,
                                    int64_t batch) {
-    int32_t rc = check_ms(h, ct, polys, l, out, batch);
-    if (rc) return rc;
-    const Context &c = *h->ctx;
-    std::vector<HostIo> in = {{(const u64 *)ct, (size_t)polys * l * c.n}};
-    const int64_t chunk = std::max<int64_t>(1, (int64_t)((size_t)4 * 1024 * 1024 / ((size_t)polys * l * c.n)));
-    return host_pipeline(h, batch, chunk, 0, in, (u64 *)out, (size_t)polys * (l - 1) * c.n,
-                         [&](Workspace &w, const std::vector<const u64 *> &d_in, u64 *d_out, int64_t items) {
-                             return launch_mod_switch(c, d_in[0], l, d_out, items * polys, w.stream);
-                         });
+    return mod_switch_down(h, ct, polys, l, out, batch, Io::Host64);
 }
-
 
 // ---------------------------------------------------------------- relinearize -> modSwitchDown, fused
 // Bfv.relinearize then Bfv.modSwitchDown on a batch in one pass (BASELINE config 3): the relinearized ciphertext stays
 // in HBM, 2 x (l-1) rows per ciphertext come back.
-int32_t hecuda_bfv_relinearize_mod_switch_down(const hecuda_context *h, const hecuda_evk *k, const uint64_t *ct3, int32_t l,
-                                               uint64_t *out, int64_t batch) {
-    int32_t rc = check_relin(h, k, ct3, l, out, batch);
-    if (rc) return rc;
+static int32_t relinearize_mod_switch_down(const hecuda_context *h, const hecuda_evk *k, const void *ct3, int32_t l,
+                                           void *out, int64_t batch, Io io) {
+    int32_t rc = check_io(h, io);
+    if (rc || (rc = check_key(h, k, true)) || (rc = check_level(h, l, "invalidCiphertext")) ||
+        (rc = check_batch(batch, {ct3, out}, "invalidCiphertext: null buffer")))
+        return rc;
     if (l < 2) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidPolyContext: modSwitchDown needs a next context (moduli_count >= 2)");
     const Context &c = *h->ctx;
     const size_t relin_words = (size_t)2 * l * c.n;
-    std::vector<HostIo> in = {{(const u64 *)ct3, (size_t)3 * l * c.n}};
-    return host_pipeline(h, batch, h->chunk, relinearize_scratch_words(c, l) + relin_words, in, (u64 *)out, (size_t)2 * (l - 1) * c.n,
-                         [&](Workspace &w, const std::vector<const u64 *> &d_in, u64 *d_out, int64_t items) {
-                             u64 *relin = w.buf[0] + relinearize_scratch_words(c, l) * (size_t)items;
-                             cudaError_t e = relinearize_chunk(c, w.buf[0], k->d_relin, d_in[0], l, relin, items, w.stream);
-                             if (e != cudaSuccess) return e;
-                             return launch_mod_switch(c, relin, l, d_out, items * 2, w.stream);
-                         });
+    return dispatch(h, io, nullptr, "relinearize_mod_switch_down", batch, h->chunk,
+                    relinearize_scratch_words(c, l) + relin_words, {{(const u64 *)ct3, (size_t)3 * l * c.n}}, out,
+                    (size_t)2 * (l - 1) * c.n, [&](const Chunk &ch) {
+                        u64 *relin = ch.scratch + relinearize_scratch_words(c, l) * (size_t)ch.items;
+                        cudaError_t e = relinearize_chunk(c, ch.scratch, k->d_relin, ch.in[0], l, relin, ch.items, ch.stream);
+                        if (e != cudaSuccess) return e;
+                        return launch_mod_switch(c, relin, l, ch.out, ch.items * 2, ch.stream);
+                    });
+}
+int32_t hecuda_bfv_relinearize_mod_switch_down(const hecuda_context *h, const hecuda_evk *k, const uint64_t *ct3, int32_t l,
+                                               uint64_t *out, int64_t batch) {
+    return relinearize_mod_switch_down(h, k, ct3, l, out, batch, Io::Host64);
 }
 
 // ---------------------------------------------------------------- multiply -> relinearize (-> modSwitchDown), fused
@@ -798,52 +810,30 @@ static cudaError_t mul_relin_chunk(const Context &c, u64 *scratch, const u64 *ke
     if (mod_switch) return launch_mod_switch(c, relin, c.L, out, items * 2, s);
     return cudaSuccess;
 }
-static int32_t check_mul_relin(const hecuda_context *h, const hecuda_evk *k, const void *lhs, const void *rhs, const void *out,
-                               int32_t mod_switch, int64_t batch) {
-    int32_t rc = check_ctx(h);
-    if (rc) return rc;
-    if (!k || !k->loaded) return fail(HECUDA_ERR_MISSING_KEY, "missingRelinearizationKey");
-    if (k->owner != h) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidContext: evaluation key belongs to another context");
+static int32_t multiply_relinearize(const hecuda_context *h, const hecuda_evk *k, const void *lhs, const void *rhs,
+                                    int32_t mod_switch, void *out, int64_t batch, Io io, void *stream = nullptr) {
+    int32_t rc = check_io(h, io);
+    if (rc || (rc = check_key(h, k, true))) return rc;
     if (mod_switch && h->ctx->L < 2)
         return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidPolyContext: modSwitchDown needs a next context (L >= 2)");
-    if (batch < 0 || (batch && (!lhs || !rhs || !out))) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidCiphertext: null buffer");
-    return HECUDA_OK;
+    if ((rc = check_batch(batch, {lhs, rhs, out}, "invalidCiphertext: null buffer"))) return rc;
+    const Context &c = *h->ctx;
+    const size_t in_words = (size_t)2 * c.L * c.n, out_words = (size_t)2 * (c.L - (mod_switch ? 1 : 0)) * c.n;
+    return dispatch(h, io, stream, "multiply_relinearize", batch, std::max<int64_t>(1, h->chunk / 2),
+                    mul_relin_scratch_words(c), {{(const u64 *)lhs, in_words}, {(const u64 *)rhs, in_words}}, out, out_words,
+                    [&](const Chunk &ch) {
+                        return mul_relin_chunk(c, ch.scratch, k->d_relin, ch.in[0], ch.in[1], mod_switch != 0, ch.out,
+                                               ch.items, ch.stream);
+                    });
 }
 int32_t hecuda_bfv_multiply_relinearize_device(const hecuda_context *h, const hecuda_evk *k, const uint64_t *lhs,
                                                const uint64_t *rhs, int32_t mod_switch, uint64_t *out, int64_t batch,
                                                void *stream) {
-    int32_t rc = check_mul_relin(h, k, lhs, rhs, out, mod_switch, batch);
-    if (rc || batch == 0) return rc;
-    const Context &c = *h->ctx;
-    const size_t in_words = (size_t)2 * c.L * c.n, out_words = (size_t)2 * (c.L - (mod_switch ? 1 : 0)) * c.n;
-    const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(h->chunk / 2, batch));
-    cudaStream_t s = (cudaStream_t)stream;
-    u64 *scratch = nullptr;
-    CK(cudaMallocAsync(&scratch, mul_relin_scratch_words(c) * (size_t)chunk * sizeof(u64), s));
-    for (int64_t done = 0; done < batch; done += chunk) {
-        const int64_t items = std::min<int64_t>(chunk, batch - done);
-        cudaError_t e = mul_relin_chunk(c, scratch, k->d_relin, (const u64 *)lhs + in_words * done, (const u64 *)rhs + in_words * done,
-                                        mod_switch != 0, (u64 *)out + out_words * done, items, s);
-        if (e != cudaSuccess) {
-            cudaFreeAsync(scratch, s);
-            return cuda_fail(e, "multiply_relinearize");
-        }
-    }
-    CK(cudaFreeAsync(scratch, s));
-    return HECUDA_OK;
+    return multiply_relinearize(h, k, lhs, rhs, mod_switch, out, batch, Io::Device, stream);
 }
 int32_t hecuda_bfv_multiply_relinearize(const hecuda_context *h, const hecuda_evk *k, const uint64_t *lhs, const uint64_t *rhs,
                                         int32_t mod_switch, uint64_t *out, int64_t batch) {
-    int32_t rc = check_mul_relin(h, k, lhs, rhs, out, mod_switch, batch);
-    if (rc) return rc;
-    const Context &c = *h->ctx;
-    const size_t in_words = (size_t)2 * c.L * c.n, out_words = (size_t)2 * (c.L - (mod_switch ? 1 : 0)) * c.n;
-    std::vector<HostIo> in = {{(const u64 *)lhs, in_words}, {(const u64 *)rhs, in_words}};
-    return host_pipeline(h, batch, std::max<int64_t>(1, h->chunk / 2), mul_relin_scratch_words(c), in, (u64 *)out, out_words,
-                         [&](Workspace &w, const std::vector<const u64 *> &d_in, u64 *d_out, int64_t items) {
-                             return mul_relin_chunk(c, w.buf[0], k->d_relin, d_in[0], d_in[1], mod_switch != 0, d_out, items,
-                                                    w.stream);
-                         });
+    return multiply_relinearize(h, k, lhs, rhs, mod_switch, out, batch, Io::Host64);
 }
 
 // ---------------------------------------------------------------- Galois (SURVEY.md 8f rank 1)
@@ -895,238 +885,172 @@ int32_t hecuda_evk_galois_device_buffer(hecuda_evk *k, uint32_t element, void **
     return HECUDA_OK;
 }
 
-static int32_t check_galois(const hecuda_context *h, const hecuda_evk *k, const uint64_t *ct, int32_t l, uint32_t element,
-                            uint64_t *out, int64_t batch, const u64 **key) {
-    int32_t rc = check_ctx(h);
-    if (rc) return rc;
-    if (!k) return fail(HECUDA_ERR_MISSING_KEY, "missingGaloisKey");
-    if (k->owner != h) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidContext: evaluation key belongs to another context");
+static int32_t apply_galois(const hecuda_context *h, const hecuda_evk *k, const void *ct, int32_t l, uint32_t element,
+                            void *out, int64_t batch, Io io, void *stream = nullptr) {
+    int32_t rc = check_io(h, io);
+    if (rc || (rc = check_key(h, k, false))) return rc;
     if (!valid_galois_element(element, h->ctx->n)) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalid Galois element");
-    if (l < 1 || l > h->ctx->L) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidCiphertext: moduli_count out of range");
-    if (batch < 0 || (batch && (!ct || !out))) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidCiphertext: null buffer");
-    hecuda_evk *km = const_cast<hecuda_evk *>(k);
-    std::lock_guard<std::mutex> g(km->mu);
-    auto it = km->galois.find(element);
-    if (it == km->galois.end()) return fail(HECUDA_ERR_MISSING_KEY, "missingGaloisElement: " + std::to_string(element));
-    *key = it->second;
-    return HECUDA_OK;
-}
-
-int32_t hecuda_bfv_apply_galois_device(const hecuda_context *h, const hecuda_evk *k, const uint64_t *ct, int32_t l,
-                                       uint32_t element, uint64_t *out, int64_t batch, void *stream) {
+    if ((rc = check_level(h, l, "invalidCiphertext")) || (rc = check_batch(batch, {ct, out}, "invalidCiphertext: null buffer")))
+        return rc;
     const u64 *key = nullptr;
-    int32_t rc = check_galois(h, k, ct, l, element, out, batch, &key);
-    if (rc) return rc;
-    if (batch == 0) return HECUDA_OK;
+    {
+        hecuda_evk *km = const_cast<hecuda_evk *>(k);
+        std::lock_guard<std::mutex> g(km->mu);
+        auto it = km->galois.find(element);
+        if (it == km->galois.end()) return fail(HECUDA_ERR_MISSING_KEY, "missingGaloisElement: " + std::to_string(element));
+        key = it->second;
+    }
     const Context &c = *h->ctx;
     const size_t words = (size_t)2 * l * c.n;
-    const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(h->chunk, batch));
-    cudaStream_t s = (cudaStream_t)stream;
-    u64 *scratch = nullptr;
-    CK(cudaMallocAsync(&scratch, galois_scratch_words(c, l) * (size_t)chunk * sizeof(u64), s));
-    for (int64_t done = 0; done < batch; done += chunk) {
-        const int64_t items = std::min<int64_t>(chunk, batch - done);
-        cudaError_t e = apply_galois_chunk(c, scratch, key, (const u64 *)ct + words * done, l, element,
-                                           (u64 *)out + words * done, items, s);
-        if (e != cudaSuccess) {
-            cudaFreeAsync(scratch, s);
-            return cuda_fail(e, "applyGalois");
-        }
-    }
-    CK(cudaFreeAsync(scratch, s));
-    return HECUDA_OK;
+    return dispatch(h, io, stream, "applyGalois", batch, h->chunk, galois_scratch_words(c, l), {{(const u64 *)ct, words}},
+                    out, words, [&](const Chunk &ch) {
+                        return apply_galois_chunk(c, ch.scratch, key, ch.in[0], l, element, ch.out, ch.items, ch.stream);
+                    });
 }
-
+int32_t hecuda_bfv_apply_galois_device(const hecuda_context *h, const hecuda_evk *k, const uint64_t *ct, int32_t l,
+                                       uint32_t element, uint64_t *out, int64_t batch, void *stream) {
+    return apply_galois(h, k, ct, l, element, out, batch, Io::Device, stream);
+}
 int32_t hecuda_bfv_apply_galois(const hecuda_context *h, const hecuda_evk *k, const uint64_t *ct, int32_t l,
                                 uint32_t element, uint64_t *out, int64_t batch) {
-    const u64 *key = nullptr;
-    int32_t rc = check_galois(h, k, ct, l, element, out, batch, &key);
-    if (rc) return rc;
-    const Context &c = *h->ctx;
-    std::vector<HostIo> in = {{(const u64 *)ct, (size_t)2 * l * c.n}};
-    return host_pipeline(h, batch, h->chunk, galois_scratch_words(c, l), in, (u64 *)out, (size_t)2 * l * c.n,
-                         [&](Workspace &w, const std::vector<const u64 *> &d_in, u64 *d_out, int64_t items) {
-                             return apply_galois_chunk(c, w.buf[0], key, d_in[0], l, element, d_out, items, w.stream);
-                         });
+    return apply_galois(h, k, ct, l, element, out, batch, Io::Host64);
 }
 
 int32_t hecuda_poly_apply_galois(const hecuda_context *h, int32_t base, int32_t eval_format, const uint64_t *in,
                                  uint64_t *out, int32_t rows, int64_t polys, uint32_t element) {
     int32_t rc = check_ctx(h);
-    if (rc) return rc;
-    if (polys < 0 || (polys && (!in || !out))) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalid data / poly_count");
+    if (rc || (rc = check_batch(polys, {in, out}, "invalid data / poly_count"))) return rc;
     if (!valid_galois_element(element, h->ctx->n)) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalid Galois element");
     NttRowMap map;
     std::string err;
     if (!make_map(*h->ctx, base, rows, map, err)) return fail(HECUDA_ERR_INVALID_ARGUMENT, err);
     const Context &c = *h->ctx;
     const size_t words = (size_t)rows * c.n;
-    std::vector<HostIo> hin = {{(const u64 *)in, words}};
-    const int64_t chunk = std::max<int64_t>(1, (int64_t)((size_t)4 * 1024 * 1024 / words));
-    return host_pipeline(h, polys, chunk, 0, hin, (u64 *)out, words,
-                         [&](Workspace &w, const std::vector<const u64 *> &d_in, u64 *d_out, int64_t items) {
-                             return eval_format ? launch_galois_eval(c, rows, element, d_in[0], d_out, items, w.stream)
-                                                : launch_galois_coeff(c, map, element, d_in[0], (int64_t)words, d_out,
-                                                                      (int64_t)words, items, w.stream);
-                         });
+    return dispatch(h, Io::Host64, nullptr, "poly_apply_galois", polys, stage_items(words), 0, {{(const u64 *)in, words}}, out,
+                    words, [&](const Chunk &k) {
+                        return eval_format ? launch_galois_eval(c, rows, element, k.in[0], k.out, k.items, k.stream)
+                                           : launch_galois_coeff(c, map, element, k.in[0], (int64_t)words, k.out,
+                                                                 (int64_t)words, k.items, k.stream);
+                    });
 }
 
 // ---------------------------------------------------------------- lazy ct x pt inner product (SURVEY.md 8f rank 2)
 
-static int32_t check_ip(const hecuda_context *h, const uint64_t *cts, int32_t polys, int32_t l, int64_t terms,
-                        const uint64_t *pts, uint64_t *out, int64_t out_count) {
-    int32_t rc = check_ctx(h);
+static int32_t inner_product_plaintexts(const hecuda_context *h, const void *cts, int32_t polys, int32_t l, int64_t terms,
+                                        const void *pts, const uint8_t *present, void *out, int64_t out_count, Io io,
+                                        void *stream = nullptr) {
+    int32_t rc = check_io(h, io);
     if (rc) return rc;
     if (polys < 1 || polys > 3) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidCiphertext: poly_count must be 1..3");
-    if (l < 1 || l > h->ctx->L) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidCiphertext: moduli_count out of range");
+    if ((rc = check_level(h, l, "invalidCiphertext"))) return rc;
     if (terms < 1) return fail(HECUDA_ERR_INVALID_ARGUMENT, "Empty ciphertexts");  // precondition, Bfv.swift:481-483
-    if (out_count < 0 || (out_count && (!cts || !pts || !out))) return fail(HECUDA_ERR_INVALID_ARGUMENT, "null buffer");
+    if ((rc = check_batch(out_count, {cts, pts, out}, "null buffer"))) return rc;
     if (h->ctx->n < 2) return fail(HECUDA_ERR_UNSUPPORTED, "degree too small");
-    return HECUDA_OK;
+    if (out_count == 0) return HECUDA_OK;
+    const Context &c = *h->ctx;
+    // the query ciphertexts (and the presence flags) are shared by every output row: a host call uploads them once
+    u64 *d_cts = nullptr;
+    unsigned char *d_present = nullptr;
+    if (io == Io::Host64) {
+        const size_t ct_words = (size_t)terms * polys * l * c.n;
+        CK(cudaMalloc(&d_cts, ct_words * sizeof(u64)));
+        cudaError_t e = upload(d_cts, cts, ct_words * sizeof(u64));
+        if (e == cudaSuccess && present) {
+            e = cudaMalloc(&d_present, (size_t)out_count * terms);
+            if (e == cudaSuccess) e = upload(d_present, present, (size_t)out_count * terms);
+        }
+        if (e != cudaSuccess) {
+            cudaFree(d_cts);
+            cudaFree(d_present);
+            return cuda_fail(e, "inner_product upload");
+        }
+        cts = d_cts;
+        present = d_present;
+    }
+    const size_t pt_words = (size_t)terms * l * c.n;
+    rc = dispatch(h, io, stream, "inner_product", out_count, stage_items(pt_words, (size_t)32 * 1024 * 1024),
+                  0, {{(const u64 *)pts, pt_words}}, out, (size_t)polys * l * c.n, [&](const Chunk &k) {
+                      const unsigned char *pr = present ? present + k.first * terms : nullptr;
+                      return launch_inner_product_plain(c, (const u64 *)cts, polys, l, terms, k.in[0], pr, k.out, k.items, k.stream);
+                  });
+    if (io == Io::Host64) {
+        cudaDeviceSynchronize();
+        cudaFree(d_cts);
+        cudaFree(d_present);
+    }
+    return rc;
 }
-
 int32_t hecuda_bfv_inner_product_plaintexts_device(const hecuda_context *h, const uint64_t *cts, int32_t polys,
                                                    int32_t l, int64_t terms, const uint64_t *pts,
                                                    const uint8_t *present, uint64_t *out, int64_t out_count,
                                                    void *stream) {
-    int32_t rc = check_ip(h, cts, polys, l, terms, pts, out, out_count);
-    if (rc) return rc;
-    cudaError_t e = launch_inner_product_plain(*h->ctx, (const u64 *)cts, polys, l, terms, (const u64 *)pts, present,
-                                               (u64 *)out, out_count, (cudaStream_t)stream);
-    if (e != cudaSuccess) return cuda_fail(e, "inner_product");
-    return HECUDA_OK;
+    return inner_product_plaintexts(h, cts, polys, l, terms, pts, present, out, out_count, Io::Device, stream);
 }
-
 int32_t hecuda_bfv_inner_product_plaintexts(const hecuda_context *h, const uint64_t *cts, int32_t polys, int32_t l,
                                             int64_t terms, const uint64_t *pts, const uint8_t *present, uint64_t *out,
                                             int64_t out_count) {
-    int32_t rc = check_ip(h, cts, polys, l, terms, pts, out, out_count);
-    if (rc) return rc;
-    if (out_count == 0) return HECUDA_OK;
-    const Context &c = *h->ctx;
-    // the query ciphertexts (and the presence flags) are shared by every output row: upload once
-    const size_t ct_words = (size_t)terms * polys * l * c.n;
-    u64 *d_cts = nullptr;
-    unsigned char *d_present = nullptr;
-    CK(cudaMalloc(&d_cts, ct_words * sizeof(u64)));
-    cudaError_t e = upload(d_cts, cts, ct_words * sizeof(u64));
-    if (e == cudaSuccess && present) {
-        e = cudaMalloc(&d_present, (size_t)out_count * terms);
-        if (e == cudaSuccess) e = upload(d_present, present, (size_t)out_count * terms);
-    }
-    if (e != cudaSuccess) {
-        cudaFree(d_cts);
-        cudaFree(d_present);
-        return cuda_fail(e, "inner_product upload");
-    }
-    const size_t pt_words = (size_t)terms * l * c.n;
-    std::vector<HostIo> in = {{(const u64 *)pts, pt_words}};
-    const int64_t chunk = std::max<int64_t>(1, (int64_t)((size_t)32 * 1024 * 1024 / pt_words));
-    int64_t done_items = 0;  // host_pipeline calls the body in order, one chunk at a time
-    rc = host_pipeline(h, out_count, chunk, 0, in, (u64 *)out, (size_t)polys * l * c.n,
-                       [&](Workspace &w, const std::vector<const u64 *> &d_in, u64 *d_out, int64_t items) {
-                           const unsigned char *pr = d_present ? d_present + done_items * terms : nullptr;
-                           done_items += items;
-                           return launch_inner_product_plain(c, d_cts, polys, l, terms, d_in[0], pr, d_out, items, w.stream);
-                       });
-    cudaDeviceSynchronize();
-    cudaFree(d_cts);
-    cudaFree(d_present);
-    return rc;
+    return inner_product_plaintexts(h, cts, polys, l, terms, pts, present, out, out_count, Io::Host64);
 }
 
+static int32_t plaintext_to_eval(const hecuda_context *h, const void *plain, int32_t l, void *out, int64_t count, Io io,
+                                 void *stream = nullptr) {
+    int32_t rc = check_io(h, io);
+    if (rc || (rc = check_level(h, l, "invalidPolyContext")) || (rc = check_batch(count, {plain, out}, "null buffer")))
+        return rc;
+    const Context &c = *h->ctx;
+    return dispatch(h, io, stream, "plaintext_to_eval", count, stage_items((size_t)l * c.n), 0, {{(const u64 *)plain, (size_t)c.n}}, out,
+                    (size_t)l * c.n, [&](const Chunk &k) {
+                        return launch_plaintext_to_eval(c, k.in[0], l, k.out, k.items, k.stream);
+                    });
+}
 int32_t hecuda_plaintext_to_eval_device(const hecuda_context *h, const uint64_t *plain, int32_t l, uint64_t *out,
                                         int64_t count, void *stream) {
-    int32_t rc = check_ctx(h);
-    if (rc) return rc;
-    if (l < 1 || l > h->ctx->L) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidPolyContext: moduli_count out of range");
-    if (count < 0 || (count && (!plain || !out))) return fail(HECUDA_ERR_INVALID_ARGUMENT, "null buffer");
-    cudaError_t e = launch_plaintext_to_eval(*h->ctx, (const u64 *)plain, l, (u64 *)out, count, (cudaStream_t)stream);
-    if (e != cudaSuccess) return cuda_fail(e, "plaintext_to_eval");
-    return HECUDA_OK;
+    return plaintext_to_eval(h, plain, l, out, count, Io::Device, stream);
 }
-
 int32_t hecuda_plaintext_to_eval(const hecuda_context *h, const uint64_t *plain, int32_t l, uint64_t *out,
                                  int64_t count) {
-    int32_t rc = check_ctx(h);
-    if (rc) return rc;
-    if (l < 1 || l > h->ctx->L) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidPolyContext: moduli_count out of range");
-    if (count < 0 || (count && (!plain || !out))) return fail(HECUDA_ERR_INVALID_ARGUMENT, "null buffer");
-    const Context &c = *h->ctx;
-    std::vector<HostIo> in = {{(const u64 *)plain, (size_t)c.n}};
-    const int64_t chunk = std::max<int64_t>(1, (int64_t)((size_t)4 * 1024 * 1024 / ((size_t)l * c.n)));
-    return host_pipeline(h, count, chunk, 0, in, (u64 *)out, (size_t)l * c.n,
-                         [&](Workspace &w, const std::vector<const u64 *> &d_in, u64 *d_out, int64_t items) {
-                             return launch_plaintext_to_eval(c, d_in[0], l, d_out, items, w.stream);
-                         });
+    return plaintext_to_eval(h, plain, l, out, count, Io::Host64);
 }
 
 // ---------------------------------------------------------------- ct x ct inner product (SURVEY.md 8f rank 2)
 
-static int32_t check_ipc(const hecuda_context *h, const uint64_t *lhs, const uint64_t *rhs, uint64_t *out, int64_t pairs,
-                         int64_t groups) {
-    int32_t rc = check_ctx(h);
+static int32_t inner_product(const hecuda_context *h, const void *lhs, const void *rhs, void *out, int64_t pairs,
+                             int64_t groups, Io io, void *stream = nullptr) {
+    int32_t rc = check_io(h, io);
     if (rc) return rc;
     if (pairs < 1) return fail(HECUDA_ERR_INVALID_ARGUMENT, "Empty ciphertexts");
-    if (groups < 0 || (groups && (!lhs || !rhs || !out))) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidCiphertext: null buffer");
+    if ((rc = check_batch(groups, {lhs, rhs, out}, "invalidCiphertext: null buffer"))) return rc;
     if (h->ctx->n < 2) return fail(HECUDA_ERR_UNSUPPORTED, "degree too small");
-    return HECUDA_OK;
-}
-
-int32_t hecuda_bfv_inner_product_device(const hecuda_context *h, const uint64_t *lhs, const uint64_t *rhs, uint64_t *out,
-                                        int64_t pairs, int64_t groups, void *stream) {
-    int32_t rc = check_ipc(h, lhs, rhs, out, pairs, groups);
-    if (rc) return rc;
-    if (groups == 0) return HECUDA_OK;
-    const Context &c = *h->ctx;
-    const size_t in_words = (size_t)pairs * 2 * c.L * c.n, out_words = (size_t)3 * c.L * c.n;
-    const int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(std::max<int64_t>(1, h->chunk / pairs), groups));
-    cudaStream_t s = (cudaStream_t)stream;
-    u64 *scratch = nullptr;
-    CK(cudaMallocAsync(&scratch, inner_product_scratch_words(c, pairs) * (size_t)chunk * sizeof(u64), s));
-    for (int64_t done = 0; done < groups; done += chunk) {
-        const int64_t g = std::min<int64_t>(chunk, groups - done);
-        cudaError_t e = inner_product_chunk(c, scratch, (const u64 *)lhs + in_words * done, (const u64 *)rhs + in_words * done,
-                                            pairs, (u64 *)out + out_words * done, g, s);
-        if (e != cudaSuccess) {
-            cudaFreeAsync(scratch, s);
-            return cuda_fail(e, "innerProduct");
-        }
-    }
-    CK(cudaFreeAsync(scratch, s));
-    return HECUDA_OK;
-}
-
-int32_t hecuda_bfv_inner_product(const hecuda_context *h, const uint64_t *lhs, const uint64_t *rhs, uint64_t *out,
-                                 int64_t pairs, int64_t groups) {
-    int32_t rc = check_ipc(h, lhs, rhs, out, pairs, groups);
-    if (rc) return rc;
     const Context &c = *h->ctx;
     const size_t in_words = (size_t)pairs * 2 * c.L * c.n;
-    std::vector<HostIo> in = {{(const u64 *)lhs, in_words}, {(const u64 *)rhs, in_words}};
-    const int64_t chunk = std::max<int64_t>(1, h->chunk / pairs);
-    return host_pipeline(h, groups, chunk, inner_product_scratch_words(c, pairs), in, (u64 *)out, (size_t)3 * c.L * c.n,
-                         [&](Workspace &w, const std::vector<const u64 *> &d_in, u64 *d_out, int64_t g) {
-                             return inner_product_chunk(c, w.buf[0], d_in[0], d_in[1], pairs, d_out, g, w.stream);
-                         });
+    return dispatch(h, io, stream, "innerProduct", groups, std::max<int64_t>(1, h->chunk / pairs),
+                    inner_product_scratch_words(c, pairs), {{(const u64 *)lhs, in_words}, {(const u64 *)rhs, in_words}},
+                    out, (size_t)3 * c.L * c.n, [&](const Chunk &k) {
+                        return inner_product_chunk(c, k.scratch, k.in[0], k.in[1], pairs, k.out, k.items, k.stream);
+                    });
+}
+int32_t hecuda_bfv_inner_product_device(const hecuda_context *h, const uint64_t *lhs, const uint64_t *rhs, uint64_t *out,
+                                        int64_t pairs, int64_t groups, void *stream) {
+    return inner_product(h, lhs, rhs, out, pairs, groups, Io::Device, stream);
+}
+int32_t hecuda_bfv_inner_product(const hecuda_context *h, const uint64_t *lhs, const uint64_t *rhs, uint64_t *out,
+                                 int64_t pairs, int64_t groups) {
+    return inner_product(h, lhs, rhs, out, pairs, groups, Io::Host64);
 }
 
 int32_t hecuda_poly_multiply_power_of_x(const hecuda_context *h, int32_t base, const uint64_t *in, uint64_t *out,
                                         int32_t rows, int64_t polys, int64_t power) {
     int32_t rc = check_ctx(h);
-    if (rc) return rc;
-    if (polys < 0 || (polys && (!in || !out))) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalid data / poly_count");
+    if (rc || (rc = check_batch(polys, {in, out}, "invalid data / poly_count"))) return rc;
     NttRowMap map;
     std::string err;
     if (!make_map(*h->ctx, base, rows, map, err)) return fail(HECUDA_ERR_INVALID_ARGUMENT, err);
     const Context &c = *h->ctx;
     const size_t words = (size_t)rows * c.n;
-    std::vector<HostIo> hin = {{(const u64 *)in, words}};
-    const int64_t chunk = std::max<int64_t>(1, (int64_t)((size_t)4 * 1024 * 1024 / words));
-    return host_pipeline(h, polys, chunk, 0, hin, (u64 *)out, words,
-                         [&](Workspace &w, const std::vector<const u64 *> &d_in, u64 *d_out, int64_t items) {
-                             return launch_multiply_power_of_x(c, map, power, d_in[0], d_out, items, w.stream);
-                         });
+    return dispatch(h, Io::Host64, nullptr, "multiply_power_of_x", polys, stage_items(words), 0, {{(const u64 *)in, words}}, out, words,
+                    [&](const Chunk &k) {
+                        return launch_multiply_power_of_x(c, map, power, k.in[0], k.out, k.items, k.stream);
+                    });
 }
 
 uint64_t hecuda_kernel_launch_count(void) { return g_kernel_launches.load(); }
@@ -1135,29 +1059,14 @@ uint64_t hecuda_kernel_launch_count(void) { return g_kernel_launches.load(); }
 // ---------------------------------------------------------------- Bfv<UInt32>: uint32 buffers at the boundary
 // (the reference's second scalar type, HeScheme.swift / Scalar.swift:498-511).  Same layouts as the uint64 entry points;
 // the context must have been made by hecuda_context_create_u32 (its m~, gamma and Bsk).
-static int32_t need_word32(const hecuda_context *h) {
-    if (!h || !h->ctx) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidContext: null context");
-    if (h->ctx->word_bits != 32) return fail(HECUDA_ERR_INVALID_ARGUMENT, "invalidContext: not a Bfv<UInt32> context (hecuda_context_create_u32)");
-    return HECUDA_OK;
-}
 int32_t hecuda_u32_ntt_forward(const hecuda_context *h, int32_t base, uint32_t *data, int32_t rows, int64_t polys) {
-    int32_t rc = need_word32(h);
-    if (rc) return rc;
-    Io32Scope scope;
-    return hecuda_ntt_forward(h, base, reinterpret_cast<uint64_t *>(data), rows, polys);
+    return ntt(h, base, data, rows, polys, false, Io::Host32);
 }
 int32_t hecuda_u32_ntt_inverse(const hecuda_context *h, int32_t base, uint32_t *data, int32_t rows, int64_t polys) {
-    int32_t rc = need_word32(h);
-    if (rc) return rc;
-    Io32Scope scope;
-    return hecuda_ntt_inverse(h, base, reinterpret_cast<uint64_t *>(data), rows, polys);
+    return ntt(h, base, data, rows, polys, true, Io::Host32);
 }
 int32_t hecuda_u32_bfv_multiply(const hecuda_context *h, const uint32_t *lhs, const uint32_t *rhs, uint32_t *out, int64_t batch) {
-    int32_t rc = need_word32(h);
-    if (rc) return rc;
-    Io32Scope scope;
-    return hecuda_bfv_multiply(h, reinterpret_cast<const uint64_t *>(lhs), reinterpret_cast<const uint64_t *>(rhs),
-                               reinterpret_cast<uint64_t *>(out), batch);
+    return multiply(h, lhs, rhs, out, batch, Io::Host32);
 }
 int32_t hecuda_u32_evk_create(const hecuda_context *h, const uint32_t *relin_key, hecuda_evk **out) {
     int32_t rc = need_word32(h);
@@ -1170,33 +1079,19 @@ int32_t hecuda_u32_evk_create(const hecuda_context *h, const uint32_t *relin_key
 }
 int32_t hecuda_u32_bfv_relinearize(const hecuda_context *h, const hecuda_evk *evk, const uint32_t *ct3, int32_t l, uint32_t *out,
                                    int64_t batch) {
-    int32_t rc = need_word32(h);
-    if (rc) return rc;
-    Io32Scope scope;
-    return hecuda_bfv_relinearize(h, evk, reinterpret_cast<const uint64_t *>(ct3), l, reinterpret_cast<uint64_t *>(out), batch);
+    return relinearize(h, evk, ct3, l, out, batch, Io::Host32);
 }
 int32_t hecuda_u32_bfv_mod_switch_down(const hecuda_context *h, const uint32_t *ct, int32_t polys, int32_t l, uint32_t *out,
                                        int64_t batch) {
-    int32_t rc = need_word32(h);
-    if (rc) return rc;
-    Io32Scope scope;
-    return hecuda_bfv_mod_switch_down(h, reinterpret_cast<const uint64_t *>(ct), polys, l, reinterpret_cast<uint64_t *>(out), batch);
+    return mod_switch_down(h, ct, polys, l, out, batch, Io::Host32);
 }
 int32_t hecuda_u32_bfv_multiply_relinearize(const hecuda_context *h, const hecuda_evk *evk, const uint32_t *lhs, const uint32_t *rhs,
                                             int32_t mod_switch, uint32_t *out, int64_t batch) {
-    int32_t rc = need_word32(h);
-    if (rc) return rc;
-    Io32Scope scope;
-    return hecuda_bfv_multiply_relinearize(h, evk, reinterpret_cast<const uint64_t *>(lhs), reinterpret_cast<const uint64_t *>(rhs),
-                                           mod_switch, reinterpret_cast<uint64_t *>(out), batch);
+    return multiply_relinearize(h, evk, lhs, rhs, mod_switch, out, batch, Io::Host32);
 }
 int32_t hecuda_u32_bfv_relinearize_mod_switch_down(const hecuda_context *h, const hecuda_evk *evk, const uint32_t *ct3, int32_t l,
                                                    uint32_t *out, int64_t batch) {
-    int32_t rc = need_word32(h);
-    if (rc) return rc;
-    Io32Scope scope;
-    return hecuda_bfv_relinearize_mod_switch_down(h, evk, reinterpret_cast<const uint64_t *>(ct3), l,
-                                                  reinterpret_cast<uint64_t *>(out), batch);
+    return relinearize_mod_switch_down(h, evk, ct3, l, out, batch, Io::Host32);
 }
 int32_t hecuda_u32_evk_set_galois_key(hecuda_evk *evk, uint32_t element, const uint32_t *key) {
     if (!evk || !key) return fail(HECUDA_ERR_INVALID_ARGUMENT, "null argument");
@@ -1207,30 +1102,17 @@ int32_t hecuda_u32_evk_set_galois_key(hecuda_evk *evk, uint32_t element, const u
 }
 int32_t hecuda_u32_bfv_apply_galois(const hecuda_context *h, const hecuda_evk *evk, const uint32_t *ct, int32_t l, uint32_t element,
                                     uint32_t *out, int64_t batch) {
-    int32_t rc = need_word32(h);
-    if (rc) return rc;
-    Io32Scope scope;
-    return hecuda_bfv_apply_galois(h, evk, reinterpret_cast<const uint64_t *>(ct), l, element, reinterpret_cast<uint64_t *>(out), batch);
+    return apply_galois(h, evk, ct, l, element, out, batch, Io::Host32);
 }
 int32_t hecuda_u32_bfv_inner_product(const hecuda_context *h, const uint32_t *lhs, const uint32_t *rhs, uint32_t *out, int64_t pairs,
                                      int64_t groups) {
-    int32_t rc = need_word32(h);
-    if (rc) return rc;
-    Io32Scope scope;
-    return hecuda_bfv_inner_product(h, reinterpret_cast<const uint64_t *>(lhs), reinterpret_cast<const uint64_t *>(rhs),
-                                    reinterpret_cast<uint64_t *>(out), pairs, groups);
+    return inner_product(h, lhs, rhs, out, pairs, groups, Io::Host32);
 }
 int32_t hecuda_u32_rnstool_lift_q_to_qbsk(const hecuda_context *h, const uint32_t *polys, uint32_t *out, int64_t count) {
-    int32_t rc = need_word32(h);
-    if (rc) return rc;
-    Io32Scope scope;
-    return hecuda_rnstool_lift_q_to_qbsk(h, reinterpret_cast<const uint64_t *>(polys), reinterpret_cast<uint64_t *>(out), count);
+    return lift_q_to_qbsk(h, polys, out, count, Io::Host32);
 }
 int32_t hecuda_u32_rnstool_floor_qbsk_to_q(const hecuda_context *h, const uint32_t *polys, uint32_t *out, int64_t count) {
-    int32_t rc = need_word32(h);
-    if (rc) return rc;
-    Io32Scope scope;
-    return hecuda_rnstool_floor_qbsk_to_q(h, reinterpret_cast<const uint64_t *>(polys), reinterpret_cast<uint64_t *>(out), count);
+    return floor_qbsk_to_q(h, polys, out, count, Io::Host32);
 }
 
 }  // extern "C"

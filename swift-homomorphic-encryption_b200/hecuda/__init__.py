@@ -169,8 +169,8 @@ def _check(rc: int):
         raise HeError(rc, (load_library().hecuda_last_error() or b"").decode())
 
 
-def _host(a) -> np.ndarray:
-    return np.ascontiguousarray(np.asarray(a, dtype=np.uint64))
+def _host(a, dtype=np.uint64) -> np.ndarray:
+    return np.ascontiguousarray(np.asarray(a, dtype=dtype))
 
 
 def _ptr(a: np.ndarray):
@@ -315,6 +315,8 @@ class Context:
 class EvaluationKey:
     """EvaluationKey<Bfv<UInt64>> holding the relinearization key (Keys.swift:66-99,222)."""
 
+    _dtype, _prefix = np.uint64, "hecuda_"  # key words and entry points of this width
+
     def __init__(self, context: Context, relinearizationKey=None):
         self.context = context
         self.galoisElements = []  # EvaluationKey.config.galoisElements
@@ -322,19 +324,20 @@ class EvaluationKey:
         if relinearizationKey is None:
             _check(load_library().hecuda_evk_create_empty(context._h, C.byref(h)))
         else:
-            key = _host(relinearizationKey)
-            K = context.L + 1
-            if key.size != context.L * 2 * K * context.degree:
-                raise HeError(-1, "invalidContext: relinearization key must be L x 2 x (L+1) x N")
-            _check(load_library().hecuda_evk_create(context._h, _ptr(key), C.byref(h)))
+            key = self._key(relinearizationKey, "relinearization")
+            _check(getattr(load_library(), self._prefix + "evk_create")(context._h, _ptr(key), C.byref(h)))
         self._h = h
 
-    def setGaloisKey(self, element: int, key):
-        """GaloisKey.keys[element] (Keys.swift:150-163): (L, 2, L+1, N) uint64, Eval format."""
-        k = _host(key)
+    def _key(self, key, kind: str) -> np.ndarray:
+        k = _host(key, self._dtype)
         if k.size != self.context.L * 2 * (self.context.L + 1) * self.context.degree:
-            raise HeError(-1, "invalidContext: Galois key must be L x 2 x (L+1) x N")
-        _check(load_library().hecuda_evk_set_galois_key(self._h, element, _ptr(k)))
+            raise HeError(-1, f"invalidContext: {kind} key must be L x 2 x (L+1) x N")
+        return k
+
+    def setGaloisKey(self, element: int, key):
+        """GaloisKey.keys[element] (Keys.swift:150-163): (L, 2, L+1, N), Eval format."""
+        k = self._key(key, "Galois")
+        _check(getattr(load_library(), self._prefix + "evk_set_galois_key")(self._h, int(element), _ptr(k)))
         if element not in self.galoisElements:
             self.galoisElements.append(int(element))
 
@@ -363,96 +366,166 @@ class EvaluationKey:
             pass
 
 
-class Bfv:
-    """enum Bfv<UInt64>: HeScheme -- the hot-path statics (Bfv/Bfv.swift:20), batched over a leading axis."""
+class EvaluationKey32(EvaluationKey):
+    """EvaluationKey<Bfv<UInt32>>: the keys as uint32 (L x 2 x (L+1) x N, Eval)."""
 
-    @staticmethod
-    def mulAssign(context: Context, lhs, rhs, out=None):
+    _dtype, _prefix = np.uint32, "hecuda_u32_"
+
+    def __init__(self, context: Context, relin_key):
+        super().__init__(context, relin_key)
+
+
+class _BfvOps:
+    """The Bfv methods that have a uint64 (hecuda_*) and a uint32 (hecuda_u32_*) entry point, written once: Bfv binds
+    them to uint64 arrays, Bfv32 to uint32 arrays.  The array shapes are checked here, before the library reads or
+    writes them."""
+
+    _dtype, _prefix = np.uint64, "hecuda_"
+
+    @classmethod
+    def _call(cls, name: str, *args):
+        _check(getattr(load_library(), cls._prefix + name)(*args))
+
+    @classmethod
+    def _out(cls, out, shape):
+        return np.empty(shape, dtype=cls._dtype) if out is None else out
+
+    @classmethod
+    def mulAssign(cls, context: Context, lhs, rhs, out=None):
         """Bfv.mulAssign (Bfv+Multiply.swift:18-21): (batch, 2, L, N) x (batch, 2, L, N) -> (batch, 3, L, N)."""
-        a, b = _host(lhs), _host(rhs)
+        a, b = _host(lhs, cls._dtype), _host(rhs, cls._dtype)
         shape = (2, context.L, context.degree)
         if a.shape[-3:] != shape or b.shape != a.shape:
             raise HeError(-1, f"invalidCiphertext: expected (..., 2, {context.L}, {context.degree}), got {a.shape} and {b.shape}")
         batch = int(np.prod(a.shape[:-3], dtype=np.int64))
-        if out is None:
-            out = np.empty(a.shape[:-3] + (3, context.L, context.degree), dtype=np.uint64)
-        _check(load_library().hecuda_bfv_multiply(context._h, _ptr(a), _ptr(b), _ptr(out), batch))
+        out = cls._out(out, a.shape[:-3] + (3, context.L, context.degree))
+        cls._call("bfv_multiply", context._h, _ptr(a), _ptr(b), _ptr(out), batch)
         return out
 
-    @staticmethod
-    def relinearizeModSwitchDown(context: Context, ciphertext, key: EvaluationKey, out=None):
+    @classmethod
+    def relinearizeModSwitchDown(cls, context: Context, ciphertext, key: EvaluationKey, out=None):
         """relinearize + modSwitchDown in one pass (hecuda_bfv_relinearize_mod_switch_down): (batch, 3, l, N) -> (batch, 2, l-1, N)."""
-        c = _host(ciphertext)
+        c = _host(ciphertext, cls._dtype)
         if c.ndim < 3 or c.shape[-3] != 3 or c.shape[-1] != context.degree:
             raise HeError(-1, "invalidCiphertext: ciphertext must have three polys when relinearizing")
         if key is None:
             raise HeError(-5, "missingRelinearizationKey")
         l = c.shape[-2]
         batch = int(np.prod(c.shape[:-3], dtype=np.int64))
-        if out is None:
-            out = np.empty(c.shape[:-3] + (2, l - 1, context.degree), dtype=np.uint64)
-        _check(load_library().hecuda_bfv_relinearize_mod_switch_down(context._h, key._h, _ptr(c), l, _ptr(out), batch))
+        out = cls._out(out, c.shape[:-3] + (2, l - 1, context.degree))
+        cls._call("bfv_relinearize_mod_switch_down", context._h, key._h, _ptr(c), l, _ptr(out), batch)
         return out
 
-    @staticmethod
-    def mulRelinearize(context: Context, lhs, rhs, key: EvaluationKey, modSwitchDown: bool = False, out=None):
+    @classmethod
+    def mulRelinearize(cls, context: Context, lhs, rhs, key: EvaluationKey, modSwitchDown: bool = False, out=None):
         """mulAssign + relinearize (+ modSwitchDown) in one pass (hecuda_bfv_multiply_relinearize): (batch, 2, L, N) x2 ->
         (batch, 2, L, N) or (batch, 2, L-1, N).  Same residues as the separate calls."""
-        a, b = _host(lhs), _host(rhs)
+        a, b = _host(lhs, cls._dtype), _host(rhs, cls._dtype)
         L, n = context.L, context.degree
         if a.shape != b.shape or a.shape[-3:] != (2, L, n):
             raise HeError(-1, "invalidCiphertext: multiply takes top-level two-polynomial ciphertexts")
         if key is None:
             raise HeError(-5, "missingRelinearizationKey")
         rows = L - 1 if modSwitchDown else L
-        if out is None:
-            out = np.empty(a.shape[:-3] + (2, rows, n), dtype=np.uint64)
-        _check(load_library().hecuda_bfv_multiply_relinearize(context._h, key._h, _ptr(a), _ptr(b), 1 if modSwitchDown else 0,
-                                                              _ptr(out), a.size // (2 * L * n)))
+        out = cls._out(out, a.shape[:-3] + (2, rows, n))
+        cls._call("bfv_multiply_relinearize", context._h, key._h, _ptr(a), _ptr(b), 1 if modSwitchDown else 0, _ptr(out),
+                  a.size // (2 * L * n))
         return out
 
-    @staticmethod
-    def relinearize(context: Context, ciphertext, key: EvaluationKey, out=None):
+    @classmethod
+    def relinearize(cls, context: Context, ciphertext, key: EvaluationKey, out=None):
         """Bfv.relinearize (Bfv.swift:201-219): (batch, 3, l, N) -> (batch, 2, l, N)."""
-        c = _host(ciphertext)
+        c = _host(ciphertext, cls._dtype)
         if c.ndim < 3 or c.shape[-3] != 3 or c.shape[-1] != context.degree:
             raise HeError(-1, "invalidCiphertext: ciphertext must have three polys when relinearizing")
         if key is None:
             raise HeError(-5, "missingRelinearizationKey")
         l = c.shape[-2]
         batch = int(np.prod(c.shape[:-3], dtype=np.int64))
-        if out is None:
-            out = np.empty(c.shape[:-3] + (2, l, context.degree), dtype=np.uint64)
-        _check(load_library().hecuda_bfv_relinearize(context._h, key._h, _ptr(c), l, _ptr(out), batch))
+        out = cls._out(out, c.shape[:-3] + (2, l, context.degree))
+        cls._call("bfv_relinearize", context._h, key._h, _ptr(c), l, _ptr(out), batch)
         return out
 
-    @staticmethod
-    def modSwitchDown(context: Context, ciphertext, out=None):
+    @classmethod
+    def modSwitchDown(cls, context: Context, ciphertext, out=None):
         """Bfv.modSwitchDown (Bfv.swift:163-171): (batch, polys, l, N) -> (batch, polys, l-1, N)."""
-        c = _host(ciphertext)
+        c = _host(ciphertext, cls._dtype)
         if c.ndim < 3 or c.shape[-1] != context.degree:
             raise HeError(-1, "invalidCiphertext")
         polys, l = c.shape[-3], c.shape[-2]
         batch = int(np.prod(c.shape[:-3], dtype=np.int64))
-        if out is None:
-            out = np.empty(c.shape[:-3] + (polys, l - 1, context.degree), dtype=np.uint64)
-        _check(load_library().hecuda_bfv_mod_switch_down(context._h, _ptr(c), polys, l, _ptr(out), batch))
+        out = cls._out(out, c.shape[:-3] + (polys, l - 1, context.degree))
+        cls._call("bfv_mod_switch_down", context._h, _ptr(c), polys, l, _ptr(out), batch)
         return out
 
-    @staticmethod
-    def applyGalois(context: Context, ciphertext, element: int, key: EvaluationKey, out=None):
+    @classmethod
+    def applyGalois(cls, context: Context, ciphertext, element: int, key: EvaluationKey, out=None):
         """Bfv.applyGalois (Bfv.swift:174-198): (batch, 2, l, N) -> (batch, 2, l, N)."""
-        c = _host(ciphertext)
+        c = _host(ciphertext, cls._dtype)
         if c.ndim < 3 or c.shape[-3] != 2 or c.shape[-1] != context.degree:
             raise HeError(-1, "invalidCiphertext: ciphertext must have two polys when applying galois")
         if key is None:
             raise HeError(-5, "missingGaloisKey")
         l = c.shape[-2]
         batch = int(np.prod(c.shape[:-3], dtype=np.int64))
-        if out is None:
-            out = np.empty_like(c)
-        _check(load_library().hecuda_bfv_apply_galois(context._h, key._h, _ptr(c), l, element, _ptr(out), batch))
+        out = cls._out(out, c.shape)
+        cls._call("bfv_apply_galois", context._h, key._h, _ptr(c), l, int(element), _ptr(out), batch)
         return out
+
+    @classmethod
+    def innerProductCiphertexts(cls, context: Context, lhs, rhs):
+        """Bfv.innerProduct(_:_:) (Bfv.swift:315-361): (groups, pairs, 2, L, N) x same -> (groups, 3, L, N)."""
+        a, b = _host(lhs, cls._dtype), _host(rhs, cls._dtype)
+        if a.ndim != 5 or a.shape != b.shape or a.shape[2:] != (2, context.L, context.degree):
+            raise HeError(-1, f"invalidCiphertext: expected (groups, pairs, 2, {context.L}, {context.degree})")
+        out = np.empty((a.shape[0], 3, context.L, context.degree), dtype=cls._dtype)
+        cls._call("bfv_inner_product", context._h, _ptr(a), _ptr(b), _ptr(out), a.shape[1], a.shape[0])
+        return out
+
+    @classmethod
+    def liftQToQBsk(cls, context: Context, polys):
+        """_RnsTool.liftQToQBsk (RnsTool.swift:324-331): (..., L, N) Coeff -> (..., 2L+1, N) over [Q, Bsk]."""
+        d = _host(polys, cls._dtype)
+        L, n = context.L, context.degree
+        if d.shape[-2:] != (L, n):
+            raise HeError(-1, "invalidPolyContext: liftQToQBsk takes top-level polynomials")
+        out = np.empty(d.shape[:-2] + (2 * L + 1, n), dtype=cls._dtype)
+        cls._call("rnstool_lift_q_to_qbsk", context._h, _ptr(d), _ptr(out), d.size // (L * n))
+        return out
+
+    @classmethod
+    def floorQBskToQ(cls, context: Context, polys):
+        """_RnsTool.floorQBskToQ (RnsTool.swift:453-456): (..., 2L+1, N) Coeff over [Q, Bsk] -> (..., L, N)."""
+        d = _host(polys, cls._dtype)
+        L, n = context.L, context.degree
+        if d.shape[-2:] != (2 * L + 1, n):
+            raise HeError(-1, "invalidPolyContext: floorQBskToQ takes polynomials over [Q, Bsk]")
+        out = np.empty(d.shape[:-2] + (L, n), dtype=cls._dtype)
+        cls._call("rnstool_floor_qbsk_to_q", context._h, _ptr(d), _ptr(out), d.size // ((2 * L + 1) * n))
+        return out
+
+    @classmethod
+    def _ntt(cls, name: str, context: Context, polys, base: int):
+        d = _host(polys, cls._dtype).copy()
+        if d.ndim < 2 or d.shape[-1] != context.degree:
+            raise HeError(-1, f"invalidPolyContext: expected (..., rows, {context.degree}), got {d.shape}")
+        rows = d.shape[-2]
+        cls._call(name, context._h, base, _ptr(d), rows, d.size // (rows * context.degree))
+        return d
+
+    @classmethod
+    def forwardNtt(cls, context: Context, polys, base: int = BASE_Q):
+        """PolyRq.forwardNtt (PolyRq+Ntt.swift:230): (..., rows, N) Coeff -> Eval."""
+        return cls._ntt("ntt_forward", context, polys, base)
+
+    @classmethod
+    def inverseNtt(cls, context: Context, polys, base: int = BASE_Q):
+        """PolyRq.inverseNtt (PolyRq+Ntt.swift:541): (..., rows, N) Eval -> Coeff."""
+        return cls._ntt("ntt_inverse", context, polys, base)
+
+
+class Bfv(_BfvOps):
+    """enum Bfv<UInt64>: HeScheme -- the hot-path statics (Bfv/Bfv.swift:20), batched over a leading axis."""
 
     @staticmethod
     def polyApplyGalois(context: Context, polys, element: int, evalFormat: bool = False, base: int = BASE_Q):
@@ -491,16 +564,6 @@ class Bfv:
         out = np.empty_like(d)
         _check(load_library().hecuda_poly_multiply_power_of_x(context._h, base, _ptr(d), _ptr(out), rows,
                                                               d.size // (rows * context.degree), power))
-        return out
-
-    @staticmethod
-    def innerProductCiphertexts(context: Context, lhs, rhs):
-        """Bfv.innerProduct(_:_:) (Bfv.swift:315-361): (groups, pairs, 2, L, N) x same -> (groups, 3, L, N)."""
-        a, b = _host(lhs), _host(rhs)
-        if a.ndim != 5 or a.shape != b.shape or a.shape[2:] != (2, context.L, context.degree):
-            raise HeError(-1, f"invalidCiphertext: expected (groups, pairs, 2, {context.L}, {context.degree})")
-        out = np.empty((a.shape[0], 3, context.L, context.degree), dtype=np.uint64)
-        _check(load_library().hecuda_bfv_inner_product(context._h, _ptr(a), _ptr(b), _ptr(out), a.shape[1], a.shape[0]))
         return out
 
     @staticmethod
@@ -619,44 +682,6 @@ class Bfv:
         return out
 
     @staticmethod
-    def liftQToQBsk(context: Context, polys):
-        """_RnsTool.liftQToQBsk (RnsTool.swift:324-331): (..., L, N) Coeff -> (..., 2L+1, N) over [Q, Bsk]."""
-        d = _host(polys)
-        L, n = context.L, context.degree
-        if d.shape[-2:] != (L, n):
-            raise HeError(-1, "invalidPolyContext: liftQToQBsk takes top-level polynomials")
-        out = np.empty(d.shape[:-2] + (2 * L + 1, n), dtype=np.uint64)
-        _check(load_library().hecuda_rnstool_lift_q_to_qbsk(context._h, _ptr(d), _ptr(out), d.size // (L * n)))
-        return out
-
-    @staticmethod
-    def floorQBskToQ(context: Context, polys):
-        """_RnsTool.floorQBskToQ (RnsTool.swift:453-456): (..., 2L+1, N) Coeff over [Q, Bsk] -> (..., L, N)."""
-        d = _host(polys)
-        L, n = context.L, context.degree
-        if d.shape[-2:] != (2 * L + 1, n):
-            raise HeError(-1, "invalidPolyContext: floorQBskToQ takes polynomials over [Q, Bsk]")
-        out = np.empty(d.shape[:-2] + (L, n), dtype=np.uint64)
-        _check(load_library().hecuda_rnstool_floor_qbsk_to_q(context._h, _ptr(d), _ptr(out), d.size // ((2 * L + 1) * n)))
-        return out
-
-    @staticmethod
-    def forwardNtt(context: Context, polys, base: int = BASE_Q):
-        """PolyRq.forwardNtt (PolyRq+Ntt.swift:230): (..., rows, N) Coeff -> Eval."""
-        d = _host(polys).copy()
-        rows = d.shape[-2]
-        _check(load_library().hecuda_ntt_forward(context._h, base, _ptr(d), rows, d.size // (rows * context.degree)))
-        return d
-
-    @staticmethod
-    def inverseNtt(context: Context, polys, base: int = BASE_Q):
-        """PolyRq.inverseNtt (PolyRq+Ntt.swift:541): (..., rows, N) Eval -> Coeff."""
-        d = _host(polys).copy()
-        rows = d.shape[-2]
-        _check(load_library().hecuda_ntt_inverse(context._h, base, _ptr(d), rows, d.size // (rows * context.degree)))
-        return d
-
-    @staticmethod
     def forwardNttRows(context: Context, modulus: int, rows):
         """PolyContext.forwardNtt(dataPtr:modulus:) (PolyRq+Ntt.swift:329-347)."""
         d = _host(rows).copy()
@@ -670,123 +695,7 @@ class Bfv:
         return d
 
 
-def _host32(a) -> np.ndarray:
-    return np.ascontiguousarray(np.asarray(a, dtype=np.uint32))
-
-
-class EvaluationKey32:
-    """EvaluationKey<Bfv<UInt32>>: relinearization key as uint32 (L x 2 x K x N, Eval)."""
-
-    def setGaloisKey(self, element: int, key):
-        k = _host32(key)
-        _check(load_library().hecuda_u32_evk_set_galois_key(self._h, int(element), _ptr(k)))
-
-    def __init__(self, context: Context, relin_key):
-        h = C.c_void_p()
-        k = _host32(relin_key)
-        _check(load_library().hecuda_u32_evk_create(context._h, _ptr(k), C.byref(h)))
-        self._h = h
-
-    def close(self):
-        if self._h is not None:
-            load_library().hecuda_evk_destroy(self._h)
-            self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-
-class Bfv32:
+class Bfv32(_BfvOps):
     """The Bfv<UInt32> data path (uint32 arrays, Context(..., scalar=np.uint32)): same shapes as the Bfv methods."""
 
-    @staticmethod
-    def mulRelinearize(context: Context, lhs, rhs, key: "EvaluationKey32", modSwitchDown: bool = False):
-        a, b = _host32(lhs), _host32(rhs)
-        L, n = context.L, context.degree
-        out = np.empty(a.shape[:-3] + (2, L - 1 if modSwitchDown else L, n), dtype=np.uint32)
-        _check(load_library().hecuda_u32_bfv_multiply_relinearize(context._h, key._h, _ptr(a), _ptr(b), 1 if modSwitchDown else 0,
-                                                                  _ptr(out), a.size // (2 * L * n)))
-        return out
-
-    @staticmethod
-    def relinearizeModSwitchDown(context: Context, ciphertext, key: "EvaluationKey32"):
-        c = _host32(ciphertext)
-        l, n = c.shape[-2], context.degree
-        out = np.empty(c.shape[:-3] + (2, l - 1, n), dtype=np.uint32)
-        _check(load_library().hecuda_u32_bfv_relinearize_mod_switch_down(context._h, key._h, _ptr(c), l, _ptr(out), c.size // (3 * l * n)))
-        return out
-
-    @staticmethod
-    def applyGalois(context: Context, ciphertext, element: int, key: "EvaluationKey32"):
-        c = _host32(ciphertext)
-        l, n = c.shape[-2], context.degree
-        out = np.empty_like(c)
-        _check(load_library().hecuda_u32_bfv_apply_galois(context._h, key._h, _ptr(c), l, int(element), _ptr(out), c.size // (2 * l * n)))
-        return out
-
-    @staticmethod
-    def innerProductCiphertexts(context: Context, lhs, rhs):
-        a, b = _host32(lhs), _host32(rhs)  # (groups, pairs, 2, L, N)
-        L, n = context.L, context.degree
-        out = np.empty((a.shape[0], 3, L, n), dtype=np.uint32)
-        _check(load_library().hecuda_u32_bfv_inner_product(context._h, _ptr(a), _ptr(b), _ptr(out), a.shape[1], a.shape[0]))
-        return out
-
-    @staticmethod
-    def forwardNtt(context: Context, polys, base: int = BASE_Q):
-        d = _host32(polys).copy()
-        rows = d.shape[-2]
-        _check(load_library().hecuda_u32_ntt_forward(context._h, base, _ptr(d), rows, d.size // (rows * context.degree)))
-        return d
-
-    @staticmethod
-    def inverseNtt(context: Context, polys, base: int = BASE_Q):
-        d = _host32(polys).copy()
-        rows = d.shape[-2]
-        _check(load_library().hecuda_u32_ntt_inverse(context._h, base, _ptr(d), rows, d.size // (rows * context.degree)))
-        return d
-
-    @staticmethod
-    def mulAssign(context: Context, lhs, rhs):
-        a, b = _host32(lhs), _host32(rhs)
-        L, n = context.L, context.degree
-        if a.shape != b.shape or a.shape[-3:] != (2, L, n):
-            raise HeError(-1, "invalidCiphertext: multiply takes top-level two-polynomial ciphertexts")
-        out = np.empty(a.shape[:-3] + (3, L, n), dtype=np.uint32)
-        _check(load_library().hecuda_u32_bfv_multiply(context._h, _ptr(a), _ptr(b), _ptr(out), a.size // (2 * L * n)))
-        return out
-
-    @staticmethod
-    def relinearize(context: Context, ciphertext, key: EvaluationKey32):
-        c = _host32(ciphertext)
-        l, n = c.shape[-2], context.degree
-        out = np.empty(c.shape[:-3] + (2, l, n), dtype=np.uint32)
-        _check(load_library().hecuda_u32_bfv_relinearize(context._h, key._h, _ptr(c), l, _ptr(out), c.size // (3 * l * n)))
-        return out
-
-    @staticmethod
-    def modSwitchDown(context: Context, ciphertext):
-        c = _host32(ciphertext)
-        polys, l, n = c.shape[-3], c.shape[-2], context.degree
-        out = np.empty(c.shape[:-3] + (polys, l - 1, n), dtype=np.uint32)
-        _check(load_library().hecuda_u32_bfv_mod_switch_down(context._h, _ptr(c), polys, l, _ptr(out), c.size // (polys * l * n)))
-        return out
-
-    @staticmethod
-    def liftQToQBsk(context: Context, polys):
-        d = _host32(polys)
-        L, n = context.L, context.degree
-        out = np.empty(d.shape[:-2] + (2 * L + 1, n), dtype=np.uint32)
-        _check(load_library().hecuda_u32_rnstool_lift_q_to_qbsk(context._h, _ptr(d), _ptr(out), d.size // (L * n)))
-        return out
-
-    @staticmethod
-    def floorQBskToQ(context: Context, polys):
-        d = _host32(polys)
-        L, n = context.L, context.degree
-        out = np.empty(d.shape[:-2] + (L, n), dtype=np.uint32)
-        _check(load_library().hecuda_u32_rnstool_floor_qbsk_to_q(context._h, _ptr(d), _ptr(out), d.size // ((2 * L + 1) * n)))
-        return out
+    _dtype, _prefix = np.uint32, "hecuda_u32_"
